@@ -59,8 +59,8 @@ def workload_config(n_gpus, dtype, tokens_per_gpu=None, batch=None):
 # reference arm / cpu baseline: the oracle port of the reference modules on the host cores
 # ------------------------------------------------------------------------------------------------
 def _cpu_modules(workload):
-    """(decoder class source, kind): the UNMODIFIED reference module when /root/reference is importable in this
-    process (the build container), else the oracle port (the GPU box has no /root/reference)."""
+    """(decoder class source, kind): the UNMODIFIED reference module when SN_REFERENCE_ROOT names a checkout of the
+    original project, else the oracle port."""
     from oracle import port
     from oracle import reference_loader as rl
     if rl.available():
@@ -151,9 +151,9 @@ def run_reference(args):
         "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")},
         "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
-        "note": "reference arm on the host cores: the unmodified reference module when /root/reference is importable "
-                "(build container), else oracle/port.py (its restatement, pinned at 1e-10); train step = "
-                "train_multitask.py:377-389.  The reference is pure Python/torch: nothing to compile into oracle/_ref",
+        "note": "reference arm on the host cores: the unmodified reference module when SN_REFERENCE_ROOT names a "
+                "checkout of it, else oracle/port.py (its restatement, pinned at 1e-10); train step = "
+                "train_multitask.py:377-389.  The reference is pure Python/torch: nothing to compile",
     }
     print(json.dumps(line), file=_JSON_OUT or sys.stdout, flush=True)
 
@@ -381,11 +381,12 @@ class Workload:
         import torch
         g, tr, kw = self._pick()
         if g is not None:
-            loss, _ = g(self.cap_pin, self.feat_pin)          # pinned host -> static device buffers, then replay
+            loss, stats = g(self.cap_pin, self.feat_pin)      # pinned host -> static device buffers, then replay
         else:
             c = self.cap_pin.to(self.dev, non_blocking=True)
             f = self.feat_pin.to(self.dev, non_blocking=True)
-            loss, _ = tr.step(c, self.lens, f, **kw)
+            loss, stats = tr.step(c, self.lens, f, **kw)
+        self.last = (loss, stats)
         self.loss_pin.copy_(loss, non_blocking=True)
         torch.cuda.current_stream().synchronize()
         return float(self.loss_pin[0])
@@ -415,6 +416,39 @@ class Workload:
             self.step_e2e()
         barrier()
         return per_step, time.perf_counter() - t0
+
+
+DUMP_SAMPLE = 1 << 16      # a tensor with more elements is dumped as this many elements at fixed seeded positions
+DUMP_LIMIT = 64 << 20      # bytes, all files together
+
+
+def dump_outputs(w, out_dir):
+    """Write what the last timed step handed its caller -- the loss, the per-token stats, and the updated parameters
+    with their gradients -- as DIR/<name>.npy (float32; integer stats as float64), so that two builds of the project
+    can be compared output for output on the same seeded inputs."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    loss, stats = w.last
+    arrays = {"loss": loss}
+    arrays.update((k, v) for k, v in stats.items() if torch.is_tensor(v))
+    for n, p in w.dec.named_parameters():
+        arrays["param." + n] = p
+        if p.grad is not None:
+            arrays["grad." + n] = p.grad
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach().reshape(-1).cpu()
+        if t.numel() > DUMP_SAMPLE:
+            pick = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE]
+            t = t[pick.sort().values]
+        out[name] = t.double().numpy() if not t.is_floating_point() or t.dtype == torch.float64 else t.float().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes, more than %d" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def dp_parity_check(dev, rank, world):
@@ -587,6 +621,8 @@ def run_gpu(args):
     ops.LAUNCHES[0] = 0
     per_step, dt_e2e = w.measure(args.steps, args.warmup, world, flush, barrier)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(w, args.dump_outputs)
     launches = ops.LAUNCHES[0] if w.graphed is None else w.launches_per_step * args.steps
     # the N-GPU == 1-GPU equality check runs AFTER the timed region (a run with it in front measured 12-15 us per step
     # more at N=2 than the same run without it: its decoders / peer mappings were still around the allocator)
@@ -911,7 +947,12 @@ def main():
     ap.add_argument("--segmented", action="store_true", help="force the 3-graph (data-parallel) replay form on one GPU")
     ap.add_argument("--no-extras", action="store_true", help="skip the fp32-mode / other-config / decode sections of the line")
     ap.add_argument("--no-dp-parity", action="store_true", help="skip the N-GPU == 1-GPU equality check (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, stats, parameters, gradients; "
+                         "large tensors as a fixed seeded sample) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     global WORKLOAD, B_PER_GPU
     WORKLOAD = args.workload
     if args.batch:

@@ -21,7 +21,7 @@ SIGNATURES = {
     "sn_last_error": (c_char_p, []),
     "sn_device_info": (_I32, [_P, _P, _P, _P]),
     "sn_gather_pack_fwd": (_I32, [_P, _I64, _P, _I64, _P, _I64, _I32, _P, _P, _P, _I64, _P, _I64, _F, c_uint64, _P, _P, _I64, _P]),
-    "sn_gather_pack_bwd": (_I32, [_P, _I64, _P, _I64, _P, _I64, _I32, _P, _P, _P, _I64, _P, _I64, _F, c_uint64, _P, _P]),
+    "sn_gather_pack_bwd": (_I32, [_P, _I64, _P, _I64, _P, _I64, _I32, _P, _P, _P, _I64, _P, _I64, _F, c_uint64, _P, _I64, _P, _P, _P]),
     "sn_gemm": (_I32, [_I32, _I64, _I64, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _F, _I32, _I64, _I64, _I64, _I64, _P]),
     "sn_gemm_bf16": (_I32, [_I32, _I64, _I64, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _F, _I32, _I64, _I64, _I64, _I64, _I64, _P]),
     "sn_gemm_bf16_splitk": (_I32, [_I32, _I64, _I64, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _F, _I32, _I64, _I64, _I64, _I64, _I64, _I32, _P]),

@@ -66,12 +66,149 @@ __global__ void gather_pack_bwd_kernel(const int64_t* __restrict__ captions, int
     }
     return;
   }
-  int64_t tok = ov >= 0 ? (int64_t)ov : captions[(int64_t)b * cap_ld + (t - has_feat)];
-  float* dst = dtable + tok * E;
-  float pp = ov >= 0 ? 0.f : p;
+  // token rows: embed_*_kernel below
+}
+
+// token of packed row i (-1: the image-feature row)
+__device__ __forceinline__ int64_t packed_token(int64_t i, const int64_t* __restrict__ captions, int64_t cap_ld,
+                                                int has_feat, const int32_t* __restrict__ row_b,
+                                                const int32_t* __restrict__ row_t,
+                                                const int32_t* __restrict__ tok_override) {
+  int ov = tok_override ? tok_override[i] : -1;
+  if (ov >= 0) return ov;
+  int t = row_t[i];
+  if (has_feat && t == 0) return -1;
+  return captions[(int64_t)row_b[i] * cap_ld + (t - has_feat)];
+}
+
+// Embedding gradient without float atomics, so that the sum (and the Adam step behind it) is the same from run to run.
+// The token rows are grouped by token with a counting sort, each group is put in row order, and each group is summed
+// in fixed chunks of EB_CHUNK rows; a group longer than one chunk adds its chunk sums in chunk order.  Every kernel is
+// parallel over rows, slots or tokens: the cost grows with N (ordering a group of s rows costs s^2 compares, which
+// for the <start> / <end> groups of B rows each is B^2).
+constexpr int EB_CHUNK = 32;  // rows summed by one warp
+constexpr int EB_K = 16;      // columns per lane and pass: 512 per pass
+
+// token of every row (-1: image-feature row) and rows per token (integer atomics: the counts are exact)
+__global__ void embed_count_kernel(const int64_t* __restrict__ captions, int64_t cap_ld, int has_feat,
+                                   const int32_t* __restrict__ row_b, const int32_t* __restrict__ row_t,
+                                   const int32_t* __restrict__ tok_override, int64_t N, int32_t* __restrict__ tok32,
+                                   int32_t* __restrict__ cnt) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= N) return;
+  const int64_t t = packed_token(r, captions, cap_ld, has_feat, row_b, row_t, tok_override);
+  tok32[r] = (int32_t)t;
+  if (t >= 0) atomicAdd(cnt + t, 1);
+}
+
+// one CTA of 1024: start = exclusive scan of cnt (start[V] = token rows), cursor = start, cstart = exclusive scan of the
+// chunk count of every group longer than one chunk
+__global__ void __launch_bounds__(1024) embed_scan_kernel(const int32_t* __restrict__ cnt, int64_t V,
+                                                          int32_t* __restrict__ start, int32_t* __restrict__ cursor,
+                                                          int32_t* __restrict__ cstart) {
+  __shared__ int32_t s1[1024], s2[1024];
+  const int tid = threadIdx.x;
+  const int64_t per = (V + 1023) / 1024, lo = tid * per, hi = lo + per < V ? lo + per : V;
+  int32_t a = 0, c = 0;
+  for (int64_t v = lo; v < hi; ++v) {
+    const int32_t n = cnt[v];
+    a += n;
+    c += n > EB_CHUNK ? (n + EB_CHUNK - 1) / EB_CHUNK : 0;
+  }
+  s1[tid] = a; s2[tid] = c;
+  __syncthreads();
+  for (int off = 1; off < 1024; off <<= 1) {       // Hillis-Steele inclusive scan
+    const int32_t x = tid >= off ? s1[tid - off] : 0, y = tid >= off ? s2[tid - off] : 0;
+    __syncthreads();
+    s1[tid] += x; s2[tid] += y;
+    __syncthreads();
+  }
+  a = s1[tid] - a; c = s2[tid] - c;
+  for (int64_t v = lo; v < hi; ++v) {
+    const int32_t n = cnt[v];
+    start[v] = a; cursor[v] = a; cstart[v] = c;
+    a += n;
+    c += n > EB_CHUNK ? (n + EB_CHUNK - 1) / EB_CHUNK : 0;
+  }
+  if (tid == 1023) start[V] = s1[1023];
+}
+
+// rows into their token's group (order inside a group still arbitrary)
+__global__ void embed_place_kernel(const int32_t* __restrict__ tok32, int64_t N, int32_t* __restrict__ cursor,
+                                   int32_t* __restrict__ perm) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= N) return;
+  const int32_t t = tok32[r];
+  if (t >= 0) perm[atomicAdd(cursor + t, 1)] = (int32_t)r;
+}
+
+// row order inside every group: a row's rank is the number of smaller row indices in its group
+__global__ void embed_order_kernel(const int32_t* __restrict__ tok32, const int32_t* __restrict__ start,
+                                   const int32_t* __restrict__ perm, int64_t N, int64_t V,
+                                   int32_t* __restrict__ sorted) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= start[V]) return;
+  const int32_t r = perm[i], t = tok32[r], s = start[t], e = start[t + 1];
+  int32_t rank = 0;
+  for (int32_t j = s; j < e; ++j) rank += perm[j] < r;
+  sorted[s + rank] = r;
+}
+
+// one warp per chunk of a group: the chunk's rows in row order; a group of one chunk goes straight to dtable
+__global__ void embed_chunk_kernel(const int32_t* __restrict__ tok32, const int32_t* __restrict__ start,
+                                   const int32_t* __restrict__ cstart, const int32_t* __restrict__ sorted, int64_t V,
+                                   const int32_t* __restrict__ tok_override, const float* __restrict__ dX, int64_t ldx,
+                                   int E, float p, float inv_keep, uint64_t seed, const uint64_t* __restrict__ seed_dev,
+                                   float* __restrict__ dtable, float* __restrict__ part) {
+  if (seed_dev) seed += *seed_dev;
+  const int64_t i = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (i >= start[V]) return;
+  const int lane = threadIdx.x & 31;
+  const int32_t t = tok32[sorted[i]], s = start[t], e = start[t + 1];
+  if ((i - s) % EB_CHUNK) return;
+  const int32_t n = (int32_t)(e - i < EB_CHUNK ? e - i : EB_CHUNK);
+  const int32_t my = lane < n ? sorted[i + lane] : 0;
+  float* dst = e - s <= EB_CHUNK ? dtable + (int64_t)t * E : part + (int64_t)(cstart[t] + (i - s) / EB_CHUNK) * E;
+  for (int c0 = 0; c0 < E; c0 += 32 * EB_K) {
+    float acc[EB_K];
+#pragma unroll
+    for (int k = 0; k < EB_K; ++k) acc[k] = 0.f;
+    for (int q = 0; q < n; ++q) {
+      const int64_t j = __shfl_sync(0xffffffffu, my, q);
+      const float pp = (tok_override && tok_override[j] >= 0) ? 0.f : p;   // fed-back embeddings: no dropout
+      const float* src = dX + j * ldx;
+#pragma unroll
+      for (int k = 0; k < EB_K; ++k) {
+        const int c = c0 + k * 32 + lane;
+        if (c < E) {
+          const float sc = sn::dropout_scale(seed, (uint32_t)j, (uint32_t)c, pp, inv_keep);
+          if (sc != 0.f) acc[k] += src[c] * sc;
+        }
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < EB_K; ++k) {
+      const int c = c0 + k * 32 + lane;
+      if (c < E) {
+        if (e - s <= EB_CHUNK) dst[c] += acc[k];
+        else dst[c] = acc[k];
+      }
+    }
+  }
+}
+
+// one warp per token whose group has several chunks: chunk sums in chunk order
+__global__ void embed_combine_kernel(const int32_t* __restrict__ cnt, const int32_t* __restrict__ cstart, int64_t V,
+                                     int E, const float* __restrict__ part, float* __restrict__ dtable) {
+  const int64_t t = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (t >= V || cnt[t] <= EB_CHUNK) return;
+  const int lane = threadIdx.x & 31;
+  const int32_t nq = (cnt[t] + EB_CHUNK - 1) / EB_CHUNK;
+  const float* src = part + (int64_t)cstart[t] * E;
   for (int c = lane; c < E; c += 32) {
-    float s = sn::dropout_scale(seed, (uint32_t)row, (uint32_t)c, pp, inv_keep);
-    if (s != 0.f) atomicAdd(dst + c, src[c] * s);
+    float a = 0.f;
+    for (int32_t q = 0; q < nq; ++q) a += src[(int64_t)q * E + c];
+    dtable[t * E + c] += a;
   }
 }
 
@@ -633,15 +770,34 @@ int32_t sn_gather_pack_bwd(const int64_t* captions, int64_t cap_ld, float* dtabl
                            float* dfeatures, int64_t feat_ld, int32_t has_feat, const int32_t* row_b,
                            const int32_t* row_t, const int32_t* tok_override, int64_t N,
                            const float* dX, int64_t ldx, float p_drop, uint64_t seed, const uint64_t* seed_dev,
-                           void* stream) {
-  SN_REQUIRE(N >= 0 && E > 0 && ldx >= E, "sn_gather_pack_bwd: bad dims");
+                           int64_t V, int32_t* ws_int, float* ws_part, void* stream) {
+  SN_REQUIRE(N >= 0 && E > 0 && ldx >= E && V > 0, "sn_gather_pack_bwd: bad dims");
   SN_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "sn_gather_pack_bwd: dropout p=%f out of [0,1)", p_drop);
+  SN_REQUIRE(N < (int64_t)1 << 30, "sn_gather_pack_bwd: N=%lld rows", (long long)N);
   if (N == 0) return 0;
+  SN_REQUIRE(ws_int && ws_part, "sn_gather_pack_bwd: null work space");
+  cudaStream_t st = (cudaStream_t)stream;
   float inv_keep = 1.f / (1.f - p_drop);
-  unsigned grid = (unsigned)((N + 7) / 8);
-  gather_pack_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(captions, cap_ld, dtable, (int)E, dfeatures, feat_ld,
-                                                                 has_feat, row_b, row_t, tok_override, N, dX, ldx,
-                                                                 p_drop, inv_keep, seed, seed_dev);
+  if (has_feat && dfeatures)
+    gather_pack_bwd_kernel<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(captions, cap_ld, dtable, (int)E, dfeatures,
+                                                                     feat_ld, has_feat, row_b, row_t, tok_override, N,
+                                                                     dX, ldx, p_drop, inv_keep, seed, seed_dev);
+  int32_t* cnt = ws_int;               // layout: see sn100.h
+  int32_t* start = cnt + V;
+  int32_t* cursor = start + V + 1;
+  int32_t* cstart = cursor + V;
+  int32_t* tok32 = cstart + V;
+  int32_t* perm = tok32 + N;
+  int32_t* sorted = perm + N;
+  SN_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)V, st));
+  const unsigned g_rows = (unsigned)((N + 255) / 256), g_warps = (unsigned)((N + 7) / 8);
+  embed_count_kernel<<<g_rows, 256, 0, st>>>(captions, cap_ld, has_feat, row_b, row_t, tok_override, N, tok32, cnt);
+  embed_scan_kernel<<<1, 1024, 0, st>>>(cnt, V, start, cursor, cstart);
+  embed_place_kernel<<<g_rows, 256, 0, st>>>(tok32, N, cursor, perm);
+  embed_order_kernel<<<g_rows, 256, 0, st>>>(tok32, start, perm, N, V, sorted);
+  embed_chunk_kernel<<<g_warps, 256, 0, st>>>(tok32, start, cstart, sorted, V, tok_override, dX, ldx, (int)E, p_drop,
+                                              inv_keep, seed, seed_dev, dtable, ws_part);
+  embed_combine_kernel<<<(unsigned)((V + 7) / 8), 256, 0, st>>>(cnt, cstart, V, (int)E, ws_part, dtable);
   return sn::check_launch("sn_gather_pack_bwd");
 }
 

@@ -1,9 +1,12 @@
 // fp32 FFMA GEMM (SN_PREC_F32): the exact-fp32 arithmetic path and the validation reference for the
 // tcgen05 GEMMs.  128x128x8 tiles, 256 threads, 8x8 register micro-tiles, generic operand strides so
 // that NT / NN / TN all run without materialised transposes.
+#include <cooperative_groups.h>
 #include <cuda_bf16.h>
 
 #include "sn_common.cuh"
+
+namespace cg = cooperative_groups;
 
 namespace {
 
@@ -188,35 +191,44 @@ __global__ void __launch_bounds__(256) gemm_skinny_nt_kernel(GemmArgs g) {
   }
 }
 
-constexpr int CS_ROWS = 128;   // rows per CTA: enough CTAs to fill the machine even for narrow matrices
+constexpr int CS_CLUSTER = 8;  // CTAs per column strip, one cluster: each sums 1/8 of the rows
+constexpr int CS_LANES = 32;   // row lanes per CTA
 
-__global__ void colsum_scale_kernel(float* __restrict__ out, int64_t N, float beta) {
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < N) out[i] *= beta;
-}
-
-// grid (ceil(N/32), ceil(M/CS_ROWS)); block 32 columns x 8 row lanes; partial sums -> one atomicAdd per column
 __device__ __forceinline__ float to_f(float v) { return v; }
 __device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
 
+// grid (ceil(N/32), CS_CLUSTER); block 32 columns x CS_LANES row lanes.  The partial sums of the cluster's CTAs are
+// added by rank 0 through distributed shared memory in rank order: every summation order is fixed, so the result is
+// the same from run to run (bias gradients feed Adam, which turns last-bit differences into +-lr steps).
 template <typename TIn>
-__global__ void colsum_kernel(const TIn* __restrict__ X, int64_t M, int64_t N, int64_t ldx,
-                              float* __restrict__ out) {
-  __shared__ float part[8][33];
+__global__ void __cluster_dims__(1, CS_CLUSTER, 1) __launch_bounds__(32 * CS_LANES) colsum_kernel(const TIn* __restrict__ X, int64_t M, int64_t N,
+                                                                 int64_t ldx, float* __restrict__ out, float beta) {
+  __shared__ float part[CS_LANES][33];
+  __shared__ float tot[32];
+  cg::cluster_group cluster = cg::this_cluster();
   const int col = blockIdx.x * 32 + threadIdx.x;
-  const int64_t r0 = (int64_t)blockIdx.y * CS_ROWS;
-  const int64_t r1 = r0 + CS_ROWS < M ? r0 + CS_ROWS : M;
+  const int64_t chunk = (M + CS_CLUSTER - 1) / CS_CLUSTER;
+  const int64_t r0 = (int64_t)blockIdx.y * chunk;
+  const int64_t r1 = r0 + chunk < M ? r0 + chunk : M;
   float s = 0.f;
   if (col < N)
-    for (int64_t m = r0 + threadIdx.y; m < r1; m += 8) s += to_f(X[m * ldx + col]);
+    for (int64_t m = r0 + threadIdx.y; m < r1; m += CS_LANES) s += to_f(X[m * ldx + col]);
   part[threadIdx.y][threadIdx.x] = s;
   __syncthreads();
-  if (threadIdx.y == 0 && col < N) {
+  if (threadIdx.y == 0) {
     float t = 0.f;
 #pragma unroll
-    for (int j = 0; j < 8; ++j) t += part[j][threadIdx.x];
-    atomicAdd(out + col, t);
+    for (int j = 0; j < CS_LANES; ++j) t += part[j][threadIdx.x];
+    tot[threadIdx.x] = t;
   }
+  cluster.sync();
+  if (cluster.block_rank() == 0 && threadIdx.y == 0 && col < N) {
+    float t = 0.f;
+#pragma unroll
+    for (int r = 0; r < CS_CLUSTER; ++r) t += cluster.map_shared_rank(tot, r)[threadIdx.x];
+    out[col] = beta == 0.f ? t : beta * out[col] + t;
+  }
+  cluster.sync();   // the other CTAs' shared memory stays alive until rank 0 has read it
 }
 
 }  // namespace
@@ -264,14 +276,12 @@ int32_t colsum_launch(const TIn* X, int64_t M, int64_t N, int64_t ldx, float* ou
   SN_REQUIRE(M >= 0 && N >= 0, "sn_colsum: bad dims");
   if (N == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (beta == 0.f) {
+  if (M == 0 && beta == 0.f) {
     SN_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)N, st));
-  } else if (beta != 1.f) {
-    colsum_scale_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(out, N, beta);
+    return 0;
   }
-  if (M == 0) return sn::check_launch("sn_colsum");
-  dim3 grid((unsigned)((N + 31) / 32), (unsigned)((M + CS_ROWS - 1) / CS_ROWS)), block(32, 8);
-  colsum_kernel<TIn><<<grid, block, 0, st>>>(X, M, N, ldx, out);
+  dim3 grid((unsigned)((N + 31) / 32), CS_CLUSTER), block(32, CS_LANES);
+  colsum_kernel<TIn><<<grid, block, 0, st>>>(X, M, N, ldx, out, beta);
   return sn::check_launch("sn_colsum");
 }
 }  // namespace

@@ -200,14 +200,19 @@ def colsum_bf16(X, M, N, ldx, out, beta=0.0):
 
 def gather_pack_bwd(captions, dtable, dfeatures, has_feat, row_b, row_t, tok_override, N, dX, p_drop, seed,
                     seed_dev=None):
-    E = dtable.shape[1]
+    V, E = dtable.shape
     cap = _req(captions, torch.int64)
+    # work space of the token grouping (layout: include/sn100.h); allocated per call so that concurrent calls on
+    # different streams never share it
+    ws_int = torch.empty(4 * V + 1 + 3 * N, dtype=torch.int32, device=dX.device)
+    ws_part = torch.empty((N // 16 + 1) * E, dtype=torch.float32, device=dX.device)
     check(lib().sn_gather_pack_bwd(
         _ptr(cap), cap.stride(0), _ptr(_req(dtable)), E,
         _ptr(dfeatures) if dfeatures is not None else None,
         dfeatures.stride(0) if dfeatures is not None else 0, 1 if has_feat else 0,
         _ptr(row_b), _ptr(row_t), _ptr(tok_override) if tok_override is not None else None,
-        N, _ptr(_req(dX)), dX.stride(0), float(p_drop), ctypes.c_uint64(seed), _ptr(seed_dev), _stream()),
+        N, _ptr(_req(dX)), dX.stride(0), float(p_drop), ctypes.c_uint64(seed), _ptr(seed_dev),
+        V, _ptr(ws_int), _ptr(ws_part), _stream()),
           "sn_gather_pack_bwd")
 
 

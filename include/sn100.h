@@ -72,7 +72,9 @@ int32_t sn_gather_pack_bwd(const int64_t* captions, int64_t cap_ld, float* dtabl
                            float* dfeatures, int64_t feat_ld, int32_t has_feat,
                            const int32_t* row_b, const int32_t* row_t, const int32_t* tok_override,
                            int64_t N, const float* dX, int64_t ldx, float p_drop, uint64_t seed,
-                           const uint64_t* seed_dev, void* stream);
+                           const uint64_t* seed_dev, int64_t V, int32_t* ws_int, float* ws_part, void* stream);
+/* Deterministic: the token rows are grouped by token (V = rows of dtable) and summed in row order, without float
+   atomics.  Work space: ws_int 4*V + 1 + 3*N int32, ws_part (N/16 + 1)*E floats. */
 
 /* ---- K2: GEMM (all nn.Linear call sites: V_g/S_*_g/U_g model.py:119-150, C model.py:189-194,
  * encoder_att/decoder_att/f_beta/init_h/init_c model_att.py:59-61,192-193,283, LSTMCell's two

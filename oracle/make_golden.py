@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz by executing the UNMODIFIED reference modules on CPU.
 
-TEST INFRASTRUCTURE ONLY.  Runs in the build container only (needs /root/reference):
+TEST INFRASTRUCTURE ONLY.  Needs a checkout of the original project:
 
-    python -m oracle.make_golden
+    SN_REFERENCE_ROOT=<checkout> python -m oracle.make_golden
 
 The reference ships no golden vectors (SURVEY.md section 8c), so these files ARE the pin: they
 record what stylenet/model.py, stylenet/model_att.py, nic/model.py, nic/model_att.py and
@@ -146,7 +146,7 @@ def make_case(name, build, att, modes, sample_variants):
 
 
 def main():
-    assert rl.available(), "needs /root/reference"
+    assert rl.available(), "set SN_REFERENCE_ROOT to a checkout of the original project"
     os.makedirs(OUT, exist_ok=True)
     sty, sty_att = rl.load("stylenet"), rl.load("stylenet_att")
     nic, nic_att = rl.load("nic"), rl.load("nic_att")

@@ -1,5 +1,5 @@
-"""Generate tests/golden/seq2seq.npz from the UNMODIFIED reference seq2seq module (/root/reference/seq2seq/model.py).
-Run in the build container only:  python -m oracle.make_golden_seq2seq
+"""Generate tests/golden/seq2seq.npz from the UNMODIFIED reference seq2seq module (seq2seq/model.py of the original).
+Needs a checkout of the original project:  SN_REFERENCE_ROOT=<checkout> python -m oracle.make_golden_seq2seq
 Contents (float64): weights of a Seq2Seq(E=12, H=16, V=61, layers=2); inputs; encoder forward (TF = 1 / 0 / 0.5, coin
 stream random.seed(1234)) logits + final states + every gradient; emotion decoder forward + gradients; greedy
 sample() ids of the encoder (batch 3) and of the factual / happy paths (batch 1) with livelier weights."""

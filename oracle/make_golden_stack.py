@@ -1,8 +1,8 @@
 """Generate tests/golden/stack3.npz: the 3-layer FactoredLSTM stack (BASELINE.json configs[3]) evaluated by composing
 UNMODIFIED reference ``DecoderFactoredLSTM`` objects through ``oracle/stack.py`` (their own ``forward_step``,
-stylenet/model.py:115-155, does all the arithmetic).  TEST INFRASTRUCTURE ONLY; build container only:
+stylenet/model.py:115-155, does all the arithmetic).  TEST INFRASTRUCTURE ONLY; needs a checkout of the original:
 
-    python -m oracle.make_golden_stack
+    SN_REFERENCE_ROOT=<checkout> python -m oracle.make_golden_stack
 """
 import os
 import random
@@ -35,7 +35,7 @@ def zero_grad(layers):
 
 
 def main():
-    assert rl.available(), "needs /root/reference"
+    assert rl.available(), "set SN_REFERENCE_ROOT to a checkout of the original project"
     sty, utils = rl.load("stylenet"), rl.load("stylenet_utils")
     torch.set_default_dtype(torch.float64)
     try:

@@ -8,7 +8,7 @@ relative to the reference repository root).
 
 Pin: ``tests/test_oracle_pin.py`` checks this port against golden vectors produced by
 the unmodified reference modules (``oracle/make_golden.py`` -> ``tests/golden/*.npz``)
-and, when ``/root/reference`` is present, against the live reference.  The reference
+and, when ``SN_REFERENCE_ROOT`` names a checkout, against the live reference.  The reference
 itself ships no tests or vectors ("parity unpinned" by upstream; SURVEY.md section 8c).
 
 Semantics that matter (SURVEY.md "ten facts"):

@@ -1,8 +1,9 @@
-"""Load the UNMODIFIED reference model files from /root/reference (build container only).
+"""Load the UNMODIFIED reference model files from a checkout of the original project.
 
-TEST INFRASTRUCTURE ONLY.  The GPU box has no /root/reference: nothing that runs there
-may call this.  Used by oracle/make_golden.py (fixture generation) and by the
-``not gpu`` pin tests (skipped when the reference tree is absent).
+TEST INFRASTRUCTURE ONLY.  The checkout is not part of this repository: it is looked for in
+``oracle/_ref`` (git-ignored) or where ``SN_REFERENCE_ROOT`` points, and without it ``available()``
+is False.  Used by oracle/make_golden*.py (fixture generation) and by the live-reference tests
+(skipped when the checkout is absent; tests/golden/ holds what the original computed).
 
 One source-text shim is applied at load time (SURVEY.md section 8c):
 ``top_k_words / self.vocab_size`` -> ``//`` so that ``sample()`` indexes with integers on
@@ -14,7 +15,7 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("SN_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("SN_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 _FILES = {
     "stylenet": "stylenet/model.py",

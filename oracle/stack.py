@@ -3,7 +3,7 @@
 The reference ignores ``num_layers`` (stylenet/model.py:37), so the stack is an EXTENSION whose definition is this
 file (SURVEY.md section 8c): ``layers`` is a list of decoder objects exposing the reference's
 ``forward_step(embedded, states, mode)`` (stylenet/model.py:115-155) -- oracle-port decoders, or the UNMODIFIED
-reference ``DecoderFactoredLSTM`` objects when /root/reference is present -- composed the way
+reference ``DecoderFactoredLSTM`` objects when the original is checked out -- composed the way
 ``nn.LSTM(num_layers)`` composes cells (seq2seq/model.py:46-49):
 
     layer 0:  forward_step(x_t,            (h0, c0), mode)      embedding B / dropout / feature row of layers[0]

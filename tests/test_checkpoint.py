@@ -1,5 +1,5 @@
 """Checkpoint interchange (SURVEY.md section 8 f3), CPU: reference whole-object checkpoints (stylenet/utils.py:63-90) ->
-drop-in modules and back.  The live-reference cases are skipped where /root/reference is absent (the GPU box)."""
+drop-in modules and back.  The live-reference cases are skipped unless SN_REFERENCE_ROOT names a checkout of the original."""
 import os
 import sys
 

@@ -1,6 +1,6 @@
 """Pin the CPU oracle (oracle/port.py) against vectors produced by the unmodified reference
-modules (tests/golden/*.npz, made by oracle/make_golden.py) and, when /root/reference is
-present, against the live reference.  float64 throughout: tolerance 1e-10 relative."""
+modules (tests/golden/*.npz, made by oracle/make_golden.py) and, when SN_REFERENCE_ROOT names a
+checkout of the original project, against the live reference.  float64 throughout: tolerance 1e-10 relative."""
 import random
 
 import numpy as np
@@ -128,7 +128,36 @@ def test_port_matches_golden_decode(name):
         torch.set_default_dtype(torch.float32)
 
 
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.parametrize("name", list(CASES))
+def test_port_fp32_matches_reference_vectors(name):
+    """fp32 port == what the UNMODIFIED reference computed (tests/golden/*.npz, float64): teacher-forced logits, loss and
+    attention weights of every mode at 1e-6 -- the stored-data form of the live fp32 comparison below."""
+    att, modes = CASES[name]
+    rec = load_golden(name)
+    dec = build_port(name, rec, dtype=torch.float32)
+    dec.train()
+    cap = torch.from_numpy(rec["in.captions"])
+    lens = [int(x) for x in rec["in.lengths"]]
+    feats = torch.from_numpy(rec["in.features"]).float()
+    for mode in modes:
+        tag = "" if mode is None else "." + mode
+        kw = {} if mode is None else {"mode": mode}
+        random.seed(1234)
+        with torch.no_grad():
+            if att:
+                l1 = [l - 1 for l in lens]
+                out, alphas = dec(cap[:, :-1], l1, feats, teacher_forcing_ratio=1.0, **kw)
+                loss = port.caption_loss(out, port.pack_targets(cap[:, 1:], l1), alphas)
+                assert rel_l2(alphas, rec["tf1.alphas" + tag]) < 1e-6
+            else:
+                out = dec(cap, lens, feats, teacher_forcing_ratio=1.0, **kw)
+                loss = port.caption_loss(out, port.pack_targets(cap, lens))
+        assert out.dtype == torch.float32
+        assert rel_l2(out, rec["tf1.logits" + tag]) < 1e-6
+        assert abs(loss.item() - float(rec["tf1.loss" + tag])) < 1e-6 * abs(float(rec["tf1.loss" + tag]))
+
+
+@pytest.mark.skipif(not rl.available(), reason="reference tree not present")
 @pytest.mark.parametrize("name,mod,cls", [
     ("factored", "stylenet", "DecoderFactoredLSTM"),
     ("factored_att", "stylenet_att", "DecoderFactoredLSTMAtt"),
