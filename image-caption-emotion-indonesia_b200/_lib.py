@@ -76,6 +76,7 @@ SIGNATURES = {
     "sn_bn1d_fwd": (_I32, [_P, _I64, _I64, _P, _P, _P, _P, _F, _F, _I32, _P, _P, _P, _P]),
     "sn_bn1d_bwd": (_I32, [_P, _P, _I64, _I64, _P, _P, _P, _I32, _P, _P, _P, _P]),
     "sn_beam_step": (_I32, [_P, _I64, _I64, _I32, _I32, _I32, _I32, _I32] + [_P] * 15),
+    "sn_bleu_counts": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _I64, _P, _P]),
 }
 
 _lib = None

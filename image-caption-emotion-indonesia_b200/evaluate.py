@@ -4,9 +4,12 @@
   * ``generate``  = the per-image ``sample()`` loop of stylenet/evaluator.py:63-101,
 with everything id-level done on the device: the loss / top-5 / arg-max come out of the fused softmax kernel instead of
 five passes over the [N, V] logits on the host, and beam search runs for a whole batch of images at once
-(``sample_batch``).  Ids -> words -> BLEU stays with the caller (nltk, CPU), exactly the reference's split."""
+(``sample_batch``).  Corpus BLEU over the ids (``bleu.corpus_bleu``, nltk's semantics) runs on the device too:
+``validate(..., bleu_weights=...)`` adds it to the result, and ``generate``'s captions go to ``bleu.corpus_bleu`` once
+<start> / <end> are stripped.  Ids -> words stays with the caller."""
 import torch
 
+from .bleu import corpus_bleu
 from .packing import get_plan
 
 
@@ -15,12 +18,15 @@ def _strip(ids, start, end):
 
 
 @torch.no_grad()
-def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, attention=None):
+def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, attention=None, bleu_weights=None):
     """``batches`` yields (images_or_features, captions [B,T] int64, lengths, all_captions | None) like the reference's
     data loader (sorted by length, data_loader.py:116-145).  Returns dict(loss, top5 (percent), hypotheses,
     references, n_tokens) with the reference's definitions: loss = token-mean cross entropy averaged over batches
     weighted by tokens (AverageMeter, utils.py:93-110), top5 = accuracy(scores, targets, 5) (utils.py:127-140),
-    hypotheses = per-caption arg-max ids cut to the caption length with <start>/<end> removed."""
+    hypotheses = per-caption arg-max ids cut to the caption length with <start>/<end> removed.
+    ``bleu_weights`` (a weight tuple or a list of them): the dict also holds "bleu" =
+    ``bleu.corpus_bleu(references, hypotheses, bleu_weights)`` (train_multitask.py:341); every batch then needs its
+    all_captions, else ValueError."""
     was_training = decoder.training
     decoder.eval()
     if encoder is not None:
@@ -31,6 +37,9 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
     tot_tok = 0
     hyps, refs = [], []
     for images, captions, lengths, all_caps in batches:
+        if all_caps is None and bleu_weights is not None:
+            decoder.train(was_training)
+            raise ValueError("validate(bleu_weights=...) needs the references (all_captions) of every batch")
         feats = encoder(images) if encoder is not None else images
         lengths = [int(l) for l in lengths]
         if att:
@@ -52,8 +61,11 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
             for caps in all_caps:
                 refs.append([_strip([int(w) for w in c], start_token, end_token) for c in caps])
     decoder.train(was_training)
-    return {"loss": tot_loss / max(tot_tok, 1), "top5": 100.0 * tot_hit / max(tot_tok, 1), "hypotheses": hyps,
-            "references": refs, "n_tokens": tot_tok}
+    res = {"loss": tot_loss / max(tot_tok, 1), "top5": 100.0 * tot_hit / max(tot_tok, 1), "hypotheses": hyps,
+           "references": refs, "n_tokens": tot_tok}
+    if bleu_weights is not None:
+        res["bleu"] = corpus_bleu(refs, hyps, bleu_weights)
+    return res
 
 
 @torch.no_grad()

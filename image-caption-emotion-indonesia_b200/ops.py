@@ -700,6 +700,19 @@ def decode_cell(cell, H, R, Wx, Kx, X, group_x, bx, Wh, bh, h_prev, c_prev, src_
           "sn_decode_cell")
 
 
+def bleu_counts(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, max_sentence_len, max_group_tokens):
+    """Per-hypothesis BLEU statistics (sn_bleu_counts): int32 [n_hyp, 10], column layout in include/sn100.h.
+    Token arrays int32, offset arrays int64, all CUDA tensors (CSR: ``hyp_off`` / ``ref_group`` have n_hyp + 1 entries,
+    ``ref_off`` one more than the number of references)."""
+    n_hyp = hyp_off.numel() - 1
+    stats = torch.empty(n_hyp, 10, dtype=torch.int32, device=hyp_off.device)
+    check(lib().sn_bleu_counts(_ptr(_req(hyp_tok, torch.int32)), _ptr(_req(hyp_off, torch.int64)), n_hyp,
+                               _ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                               _ptr(_req(ref_group, torch.int64)), int(max_sentence_len), int(max_group_tokens),
+                               _ptr(_req(stats, torch.int32)), _stream()), "sn_bleu_counts")
+    return stats
+
+
 def gate_wait(flag3, timeout_us=300):
     """Queue a one-thread kernel that returns once the cluster-form reverse recurrence (given the same flag) is resident."""
     check(lib().sn_gate_wait(_ptr(_req(flag3, torch.int32)), int(timeout_us), _stream()), "sn_gate_wait")

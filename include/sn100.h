@@ -450,6 +450,29 @@ int32_t sn_bn1d_bwd(const float* x, const float* dy, int64_t B, int64_t E, const
                     const float* save_mean, const float* save_invstd, int32_t training, float* dx,
                     float* dgamma, float* dbeta, void* stream);
 
+/* ---- K10: corpus-BLEU n-gram statistics (sn_bleu.cu) -------------------------------------------------------------
+ * replaces the per-hypothesis loop of nltk's corpus_bleu -- modified_precision and closest_ref_length
+ * (nltk/translate/bleu_score.py) -- called by the reference at the end of every validation epoch
+ * (stylenet/train_multitask.py:341, evaluator.py:103).
+ * Inputs in CSR form (device memory): hypothesis i is hyp_tok[hyp_off[i] .. hyp_off[i+1]) and owns the references
+ * ref_group[i] .. ref_group[i+1]-1; reference r is ref_tok[ref_off[r] .. ref_off[r+1]).  The references of one
+ * hypothesis are contiguous.  max_sentence_len (longest hypothesis or reference, <= SN_BLEU_MAX_LEN) and
+ * max_group_tokens (largest hypothesis length + total length of its references, sizes shared memory) are computed
+ * by the caller while packing; either limit exceeded -> rc < 0 before any launch.
+ * Output stats [n_hyp, 10] int32, per hypothesis:
+ *   0..3  clipped n-gram matches, n = 1..4: sum over distinct hypothesis n-grams g of
+ *         min(count_hyp(g), max over references of count_ref(g))         (modified_precision numerator)
+ *   4..7  max(1, len_hyp - n + 1)                                         (modified_precision denominator)
+ *   8     len_hyp
+ *   9     closest reference length: minimises (|len_ref - len_hyp|, len_ref), ties -> the shorter reference
+ *         (closest_ref_length); 0 for a hypothesis without references
+ * Integer arithmetic, no atomics: exact and run-to-run identical.  Corpus totals are column sums.  A hypothesis
+ * whose sizes exceed the declared maxima gets -1 in every column. */
+#define SN_BLEU_MAX_LEN 256
+int32_t sn_bleu_counts(const int32_t* hyp_tok, const int64_t* hyp_off, int64_t n_hyp,
+                       const int32_t* ref_tok, const int64_t* ref_off, const int64_t* ref_group,
+                       int32_t max_sentence_len, int64_t max_group_tokens, int32_t* stats, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
