@@ -71,6 +71,8 @@ SIGNATURES = {
     "sn_skinny_max_rows": (_I32, []),
     "sn_skinny_linear": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _I64, _I64, _P, _P, _I64, _P, _P]),
     "sn_decode_cell": (_I32, [_I32, _I64, _I64, _P, _I64, _I64, _P, _I64, _I64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "sn_decode_cell_groups": (_I32, [_I32, _I64, _I64, _P, _I64, _P, _I64, _I64, _I64, _P, _I64, _I64, _P, _I64, _P, _P,
+                                     _P, _P, _P, _P, _P, _P, _P]),
     "sn_pool_nhwc_fwd": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P]),
     "sn_pool_nhwc_bwd": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P]),
     "sn_bn1d_fwd": (_I32, [_P, _I64, _I64, _P, _P, _P, _P, _F, _F, _I32, _P, _P, _P, _P]),

@@ -25,6 +25,52 @@ class _StepCtx:
     pass
 
 
+class StyleGroups(tuple):
+    """The style groups of a mixed-style decode call: ``(styles, counts)``, group g = ``counts[g]`` consecutive images
+    captioned in ``styles[g]``.  Hashable: it is the ``mode`` part of the session key."""
+
+    @property
+    def styles(self):
+        return self[0]
+
+    @property
+    def counts(self):
+        return self[1]
+
+
+def group_styles(modes, n_img, styles):
+    """Stable grouping of a per-image style list (``sample_batch(..., mode=[...])``) in the order of ``styles``.
+    Returns (StyleGroups, order): ``order[j]`` is the input index of the j-th image in grouped order.  Raises
+    ValueError for an empty list, a length other than ``n_img`` or an unknown style -- before any device work."""
+    if not isinstance(modes, (list, tuple)):
+        raise ValueError("mode must be a style name or a list / tuple of them, got %r" % (modes,))
+    if len(modes) == 0:
+        raise ValueError("empty style list")
+    if len(modes) != n_img:
+        raise ValueError("style list of length %d for %d images" % (len(modes), n_img))
+    for m in modes:
+        if not isinstance(m, str) or m not in styles:
+            raise ValueError("mode name wrong: %r (expected one of %s)" % (m, tuple(styles)))
+    present = [s for s in styles if s in modes]
+    order = [i for s in present for i in range(n_img) if modes[i] == s]
+    counts = tuple(sum(1 for m in modes if m == s) for s in present)
+    return StyleGroups((tuple(present), counts)), order
+
+
+def require_one_style(mode):
+    """``sample()`` captions one image in one style; a style list is ``sample_batch``'s."""
+    if isinstance(mode, (list, tuple)):
+        raise ValueError("sample() takes one style name; pass a per-image style list to sample_batch()")
+
+
+def ungroup(results, order):
+    """Results in grouped order back to input order."""
+    out = [None] * len(order)
+    for j, i in enumerate(order):
+        out[i] = results[j]
+    return out
+
+
 def _n_layers(dec):
     """Stacked decoders (stack.DecoderFactoredLSTMStack) keep one (h, c) per layer; the reference models have one."""
     return int(dec.num_layers) if getattr(dec, "_layered", False) else 1
@@ -192,9 +238,23 @@ class _DecodeSession:
         self.graph = None          # generic step (steps >= 2)
         self.calls = 0
         self.arena_version = dec.arena().version
+        # mixed styles: group g = rows [row_off[g], row_off[g+1]) in style groups.styles[g]
+        self.groups = mode if isinstance(mode, StyleGroups) else None
+        if self.groups is not None:
+            self.row_off = [0]
+            for n in self.groups.counts:
+                self.row_off.append(self.row_off[-1] + n * k)
+            self.row_off_dev = _i32(dev, self.row_off)
+            self.rows_max = max(self.groups.counts) * k
+            self.gctx = [[_StepCtx() for _ in self.groups.styles] for _ in range(L)]
+            for l in range(L):
+                for g, gc in enumerate(self.gctx[l]):
+                    gc.layer, gc.w16 = l, {}
+                    gc.XP = self.ctx.XP[self.row_off[g]:self.row_off[g + 1]]     # the group's rows of the shared XP
         # few rows (single-image beam search): matrix-vector kernels, state double-buffered (A -> B -> A ...), the beam
         # re-ordering of the state folded into the next step's read (no index_select kernels)
-        self.skinny = R <= ops.SKINNY_MAX_ROWS
+        self.skinny = R <= (ops.SKINNY_MAX_ROWS if self.groups is None else
+                            min(STYLES_SKINNY_MAX_ROWS[0], ops.SKINNY_LINEAR_MAX_ROWS))
         if self.skinny:
             self.hB, self.cB = torch.zeros(L, R, H, **f32), torch.zeros(L, R, H, **f32)
             self.flip = 0              # 0: the state is in (h, c); 1: in (hB, cB)
@@ -212,9 +272,17 @@ class _DecodeSession:
         X = self.X
         for l in range(self.L):
             self.ctx.layer = l
-            if self.L > 1:
-                self.ctx.w16 = self.__dict__.setdefault("_w16_layers", {}).setdefault(l, {})
-            dec._input_projection(self.ctx, X, self.mode, 0, R)
+            if self.groups is not None:
+                # the chain per group on its rows of XP.  Only S is the group's: the V stage (and, in bf16 mode, the V / U
+                # weight shadows) is recomputed per group -- G - 1 redundant V GEMMs per step; sharing it would need a
+                # split of _input_projection into its stages
+                for g, style in enumerate(self.groups.styles):
+                    r0, r1 = self.row_off[g], self.row_off[g + 1]
+                    dec._input_projection(self.gctx[l][g], X[r0:r1], style, 0, r1 - r0)
+            else:
+                if self.L > 1:
+                    self.ctx.w16 = self.__dict__.setdefault("_w16_layers", {}).setdefault(l, {})
+                dec._input_projection(self.ctx, X, self.mode, 0, R)
             Whh, bhh = _rw(dec, l)
             ops.recur_fwd(dec.cell, H, R, self.bs1, self.off1, 0, 1, self.ctx.XP, Whh, bhh, self.h[l], self.h_new[l], None,
                           None, None, self.c[l])
@@ -245,6 +313,15 @@ class _DecodeSession:
         src = (self.h, self.c) if self.flip == 0 else (self.hB, self.cB)
         dst = (self.hB, self.cB) if self.flip == 0 else (self.h, self.c)
         for l in range(self.L):
+            if self.groups is not None:
+                # every style group in one launch, each with the collapsed chain of its style (_collapse_styles)
+                ent = self.ctx.collapsed_groups[l]
+                Whh, bhh = _rw(dec, l)
+                ops.decode_cell_groups(dec.cell, dec.hidden_size, self.row_off_dev, self.rows_max, ent["Wc"], X.shape[1],
+                                       X, 0, ent["bc"], Whh, bhh, src[0][l], src[1][l], st.src_row, dst[0][l],
+                                       dst[1][l], x_rows=rows if l == 0 else None)
+                X = dst[0][l]
+                continue
             kw = {"layer": l} if l else {}
             if l == 0 and rows is not None:
                 kw["x_rows"] = rows
@@ -287,6 +364,12 @@ class _DecodeSession:
 
 
 COLLAPSE_CHAIN = [True]       # few-row decode: collapse the factored chain once per call (DecoderFactoredLSTM._collapse_chain)
+# mixed-style decode (sample_batch with a style list): up to this many rows (images x k) on the matrix-vector kernels
+# (sn_decode_cell_groups + the row-chunked vocabulary projection), above it on the GEMM path.  Set from bench_styles.py
+# (profiles/styles_bench_N1.jsonl, one B200 at 1000 W): the few-row path led at every size swept, 20 / 40 / 80 / 120 rows
+# (2.4 / 5.3 / 8.4 / 18.6 ms per request vs 4.7 / 8.3 / 11.8 / 20.8 on the GEMM path), its lead shrinking to 11 % at
+# 120 rows; the cap is the largest size measured -- where the two paths cross above it is not measured
+STYLES_SKINNY_MAX_ROWS = [120]
 
 
 def _session(dec, n_img, k, mode, start_token, end_token):
@@ -305,10 +388,19 @@ def _session(dec, n_img, k, mode, start_token, end_token):
 def beam_sample(dec, features, start_token, end_token, k, mode, feed_image, sync_every=4, use_graph=None):
     """Returns a list of LongTensor [1, L_i] (one per image; the reference handles one image per call).
     ``features``: [n_img, E] (or [n_img, 1, E]); rows are independent images.
-    ``use_graph`` (default: fp32 mode): steps >= 2 replay one captured CUDA graph of the decode step."""
+    ``use_graph`` (default: fp32 mode): steps >= 2 replay one captured CUDA graph of the decode step.
+    ``mode`` a list / tuple of n_img style names (factored decoders): image i in style mode[i], one beam search over
+    the images grouped by style, results in input order."""
     emb = dec._emb()
     E = emb.weight.shape[1]
     dev = emb.weight.device
+    if isinstance(mode, (list, tuple)) and not isinstance(mode, StyleGroups):
+        from .decoders import STYLES
+        groups, order = group_styles(mode, features.numel() // E, STYLES)
+        feats = features.detach().to(dev).float().reshape(-1, E)
+        feats = feats.index_select(0, torch.tensor(order, dtype=torch.long, device=dev))
+        res = beam_sample(dec, feats, start_token, end_token, k, groups, feed_image, sync_every, use_graph)
+        return ungroup(res, order)
     ops.lib()
     dec.arena()
     feats = features.detach().to(dev).float().reshape(-1, E)
@@ -348,7 +440,10 @@ def beam_sample(dec, features, start_token, end_token, k, mode, feed_image, sync
             else:
                 restart_eager()
         sess.feats.copy_(feats)
-        if COLLAPSE_CHAIN[0] and hasattr(dec, "_collapse_chain"):
+        if sess.groups is not None:
+            for l in range(sess.L):
+                dec._collapse_styles(sess.ctx, sess.groups.styles, l)    # one Wc / bc per style, this call's weights
+        elif COLLAPSE_CHAIN[0] and hasattr(dec, "_collapse_chain"):
             # inference: U_g S_g V_g of this mode as one matrix per gate, refreshed once per call (the weights may have
             # been trained since the last one) -- a decode step is then ONE kernel in front of the vocabulary projection
             for l in range(sess.L):
@@ -380,6 +475,9 @@ def beam_sample(dec, features, start_token, end_token, k, mode, feed_image, sync
     sess.cache.clear()
     sess.ctx.w16 = {}
     sess.__dict__.pop("_w16_layers", None)
+    for gcs in sess.__dict__.get("gctx", ()):
+        for gc in gcs:
+            gc.w16 = {}
     graph = sess.graph if use_graph else None
     for step in range(1, dec.max_seq_length + 2):
         if graph is not None and step >= 2:
@@ -395,25 +493,47 @@ def beam_sample(dec, features, start_token, end_token, k, mode, feed_image, sync
 def beam_sample_att(dec, features, start_token, end_token, k, mode, sync_every=4):
     """Attention beam search (stylenet/model_att.py:307-426) for n_img images: features
     [n_img, S, S, D] (or [n_img, P, D]).  The feature map and the hoisted att1 are stored once per image;
-    live beams index them through ``row_img`` instead of expanding them k times."""
+    live beams index them through ``row_img`` instead of expanding them k times.
+    ``mode`` a list / tuple of n_img style names: image i in style mode[i].  The images are grouped by style; per group
+    the hoisted att1 comes from that style's encoder_att, and each step runs its decoder_att, the attention step and
+    the style's input projection on the group's rows, while f_beta, the recurrence and C run once over all rows."""
     emb = dec._emb()
     E = emb.weight.shape[1]
     dev = emb.weight.device
+    D, A, H = dec.feature_size, dec.attention_size, dec.hidden_size
+    order = None
+    if isinstance(mode, (list, tuple)):
+        from .decoders import STYLES
+        n_in = features.shape[0] if features.dim() >= 3 else 1
+        groups, order = group_styles(mode, n_in, STYLES)
+        styles, counts = groups.styles, groups.counts
     ops.lib()
     dec.arena()
-    D, A, H = dec.feature_size, dec.attention_size, dec.hidden_size
     feats = features.detach().to(dev).float()
     n_img = feats.shape[0] if feats.dim() >= 3 else 1
     feats = feats.reshape(n_img, -1, D).contiguous()
+    if order is not None:
+        feats = feats.index_select(0, torch.tensor(order, dtype=torch.long, device=dev))
+    else:
+        styles, counts = (mode,), (n_img,)
+    G = len(styles)
+    # group g: images [img_off[g], img_off[g+1]), rows [k * img_off[g], k * img_off[g+1])
+    img_off = [0]
+    for n in counts:
+        img_off.append(img_off[-1] + n)
     P = feats.shape[1]
-    att = dec._att_module(mode)
+    atts = [dec._att_module(s) for s in styles]
     st = BeamState(n_img, k, dec.max_seq_length, start_token, dev)
     R = st.R
     f32 = dict(dtype=torch.float32, device=dev)
     h0, c0 = dec.init_hidden_state(feats)
     h = h0.repeat_interleave(k, 0).contiguous()
     c = c0.repeat_interleave(k, 0).contiguous()
-    att1 = ops.linear_nt(feats.view(n_img * P, D), att.encoder_att.weight, att.encoder_att.bias)
+    att1 = torch.empty(n_img * P, A, **f32)
+    for g, att in enumerate(atts):
+        i0, i1 = img_off[g], img_off[g + 1]
+        ops.linear_nt(feats[i0:i1].view((i1 - i0) * P, D), att.encoder_att.weight, att.encoder_att.bias,
+                      out=att1[i0 * P:i1 * P])
     # per-row views of the per-image tensors (beams of one image share its rows)
     feats_r = feats.repeat_interleave(k, 0).contiguous()
     att1_r = att1.view(n_img, P, A).repeat_interleave(k, 0).contiguous()
@@ -427,17 +547,33 @@ def beam_sample_att(dec, features, start_token, end_token, k, mode, sync_every=4
     alpha = torch.empty(R, P, **f32)
     ctx = _StepCtx()
     ctx.XP = torch.empty(R, 4 * H, **f32)
+    gctx = []
+    for g in range(G):
+        gc = _StepCtx()
+        gc.XP = ctx.XP[k * img_off[g]:k * img_off[g + 1]]
+        gctx.append(gc)
     row_img = torch.zeros(R, dtype=torch.int32, device=dev)
     dummy_cap = torch.zeros(1, 1, dtype=torch.int64, device=dev)
     bs1, off1 = _i32(dev, [R]), _i32(dev, [0])
     Whh, bhh = dec._recurrent_weights()
-    wfull = att.full_att.weight.view(-1)
+    wfull = [att.full_att.weight.view(-1) for att in atts]
     for step in range(1, dec.max_seq_length + 2):
         ops.gather_pack_fwd(dummy_cap, emb.weight, None, False, row_img, row_img, st.prev_word, R, X, 0.0, 0)
-        ops.gemm(ops.OP_NT, h, att.decoder_att.weight, att2, R, A, H, H, H, A, bias=att.decoder_att.bias)
+        for g, att in enumerate(atts):
+            r0, r1 = k * img_off[g], k * img_off[g + 1]
+            ops.gemm(ops.OP_NT, h[r0:r1], att.decoder_att.weight, att2[r0:r1], r1 - r0, A, H, H, H, A,
+                     bias=att.decoder_att.bias)
         ops.gemm(ops.OP_NT, h, dec.f_beta.weight, gate_pre, R, D, H, H, H, D, bias=dec.f_beta.bias)
-        ops.att_step_fwd(att1_r, att2, feats_r, wfull, 0.0, gate_pre, R, P, A, D, alpha, P, X[:, E:], E + D)
-        dec._input_projection(ctx, X, mode, 0, R)
+        for g in range(G):
+            r0, r1 = k * img_off[g], k * img_off[g + 1]
+            ops.att_step_fwd(att1_r[r0:r1], att2[r0:r1], feats_r[r0:r1], wfull[g], 0.0, gate_pre[r0:r1], r1 - r0, P, A,
+                             D, alpha[r0:r1], P, X[r0:r1, E:], E + D)
+        if G == 1:
+            dec._input_projection(ctx, X, styles[0], 0, R)
+        else:
+            for g in range(G):
+                r0, r1 = k * img_off[g], k * img_off[g + 1]
+                dec._input_projection(gctx[g], X[r0:r1], styles[g], 0, r1 - r0)
         ops.recur_fwd(dec.cell, H, R, bs1, off1, 0, 1, ctx.XP, Whh, bhh, h, h_new, None, None, None, c)
         ops.gemm(ops.OP_NT, h_new, out.weight, logits, R, V, H, H, H, V, bias=out.bias)
         st.step(logits, step, end_token)
@@ -446,4 +582,5 @@ def beam_sample_att(dec, features, start_token, end_token, k, mode, sync_every=4
         c = c.index_select(0, idx)
         if sync_every and step % sync_every == 0 and int(st.n_unfinished.item()) == 0:
             break
-    return st.results()
+    res = st.results()
+    return res if order is None else ungroup(res, order)

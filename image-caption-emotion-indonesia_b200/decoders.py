@@ -1011,28 +1011,61 @@ class DecoderFactoredLSTM(_DecoderBase):
         if mode not in STYLES:
             raise ValueError("mode name wrong: %r (expected one of %s)" % (mode, STYLES))
         H, F = self.hidden_size, self.factored_size
-        Ein = self.arena().named[self._lp(layer) + "V_" + GATES[0] + ".weight"].shape[1]
-        Vc, bV = self._stack("V_", (4 * F, Ein), layer=layer), self._stack("V_", (4 * F,), bias=True, layer=layer)
-        Sc, bS = self._style_stack(mode, (4 * F, F), layer=layer), self._style_stack(mode, (4 * F,), bias=True, layer=layer)
-        Uc, bU = self._stack("U_", (4 * H, F), layer=layer), self._stack("U_", (4 * H,), bias=True, layer=layer)
+        Ein = self._chain_in(layer)
         col = ctx.__dict__.setdefault("collapsed", {})
         ent = col.get(layer)
         key = (mode, self.arena().content_key())
         if ent is not None and ent.get("key") == key:
             return ent                         # same weights as at the last call (evaluation loops): nothing to refresh
-        dev = Vc.device
         if ent is None or ent["Wc"].shape != (4 * H, Ein):
-            f32 = dict(dtype=torch.float32, device=dev)
+            f32 = dict(dtype=torch.float32, device=self.B.weight.device)
             ent = col[layer] = {"Wc": torch.empty(4 * H, Ein, **f32), "bc": torch.empty(4 * H, **f32),
                                 "SV": torch.empty(4 * F, Ein, **f32), "t": torch.empty(4 * F, **f32)}
-        with torch.no_grad():
-            ops.gemm(ops.OP_NN, Sc, Vc, ent["SV"], F, Ein, F, F, Ein, Ein, batch=4, sA=F * F, sB=F * Ein, sC=F * Ein)
-            ops.gemm(ops.OP_NN, Uc, ent["SV"], ent["Wc"], H, Ein, F, F, Ein, Ein, batch=4, sA=H * F, sB=F * Ein, sC=H * Ein)
-            ops.gemm(ops.OP_NN, Sc, bV, ent["t"], F, 1, F, F, 1, 1, batch=4, sA=F * F, sB=F, sC=F)
-            ent["t"].add_(bS)
-            ops.gemm(ops.OP_NN, Uc, ent["t"], ent["bc"], H, 1, F, F, 1, 1, batch=4, sA=H * F, sB=F, sC=H)
-            ent["bc"].add_(bU)
+        self._collapse_into(mode, layer, ent["Wc"], ent["bc"], ent["SV"], ent["t"])
         ent["mode"], ent["key"] = mode, key
+        return ent
+
+    def _chain_in(self, layer):
+        """Input width of layer ``layer``'s factored chain (E for the first layer, H above it)."""
+        return self.arena().named[self._lp(layer) + "V_" + GATES[0] + ".weight"].shape[1]
+
+    def _collapse_into(self, mode, layer, Wc, bc, SV, t):
+        """The GEMMs of ``_collapse_chain``: Wc [4H, Ein], bc [4H] of ``mode``; SV [4F, Ein] and t [4F] are scratch."""
+        H, F = self.hidden_size, self.factored_size
+        Ein = Wc.shape[1]
+        Vc, bV = self._stack("V_", (4 * F, Ein), layer=layer), self._stack("V_", (4 * F,), bias=True, layer=layer)
+        Sc, bS = self._style_stack(mode, (4 * F, F), layer=layer), self._style_stack(mode, (4 * F,), bias=True, layer=layer)
+        Uc, bU = self._stack("U_", (4 * H, F), layer=layer), self._stack("U_", (4 * H,), bias=True, layer=layer)
+        with torch.no_grad():
+            ops.gemm(ops.OP_NN, Sc, Vc, SV, F, Ein, F, F, Ein, Ein, batch=4, sA=F * F, sB=F * Ein, sC=F * Ein)
+            ops.gemm(ops.OP_NN, Uc, SV, Wc, H, Ein, F, F, Ein, Ein, batch=4, sA=H * F, sB=F * Ein, sC=H * Ein)
+            ops.gemm(ops.OP_NN, Sc, bV, t, F, 1, F, F, 1, 1, batch=4, sA=F * F, sB=F, sC=F)
+            t.add_(bS)
+            ops.gemm(ops.OP_NN, Uc, t, bc, H, 1, F, F, 1, 1, batch=4, sA=H * F, sB=F, sC=H)
+            bc.add_(bU)
+
+    def _collapse_styles(self, ctx, styles, layer=0):
+        """``_collapse_chain`` for several styles of one decode call (``sample_batch`` with a per-image style list):
+        Wc [G, 4H, Ein] / bc [G, 4H], entry g the collapsed chain of ``styles[g]`` -- the same GEMMs, so bit for bit
+        the single-style matrices.  Fixed addresses (graph-captured steps read them), refreshed in place whenever the
+        weights have changed since the last call."""
+        for mode in styles:
+            if mode not in STYLES:
+                raise ValueError("mode name wrong: %r (expected one of %s)" % (mode, STYLES))
+        H, F = self.hidden_size, self.factored_size
+        Ein, G = self._chain_in(layer), len(styles)
+        col = ctx.__dict__.setdefault("collapsed_groups", {})
+        ent = col.get(layer)
+        key = (tuple(styles), self.arena().content_key())
+        if ent is not None and ent.get("key") == key:
+            return ent
+        if ent is None or ent["Wc"].shape != (G, 4 * H, Ein):
+            f32 = dict(dtype=torch.float32, device=self.B.weight.device)
+            ent = col[layer] = {"Wc": torch.empty(G, 4 * H, Ein, **f32), "bc": torch.empty(G, 4 * H, **f32),
+                                "SV": torch.empty(4 * F, Ein, **f32), "t": torch.empty(4 * F, **f32)}
+        for g, mode in enumerate(styles):
+            self._collapse_into(mode, layer, ent["Wc"][g], ent["bc"][g], ent["SV"], ent["t"])
+        ent["key"] = key
         return ent
 
     def _small_step(self, ctx, X, mode, R, h_prev, c_prev, src_row, h_out, c_out, layer=0, x_rows=None):
@@ -1086,13 +1119,17 @@ class DecoderFactoredLSTM(_DecoderBase):
                feed_image=False):
         """Beam search with the reference's semantics (stylenet/model.py:198-294; ``feed_image=True`` is
         the app/backend/model.py:386-487 variant).  Returns LongTensor [1, L]."""
-        from .decode import beam_sample
+        from .decode import beam_sample, require_one_style
+        require_one_style(mode)
         return beam_sample(self, features, start_token, end_token, k, mode, feed_image)[0]
 
     def sample_batch(self, features, start_token, end_token, k=5, mode="factual", feed_image=False):
         """``sample()`` for every row of ``features [n_img, E]`` in one batched beam search (an addition beside the kept
         surface, SURVEY.md section 8b; replaces the per-image loop of stylenet/evaluator.py:74-81).  Returns a list of
-        LongTensor [1, L_i], element i identical to ``sample(features[i:i+1], ...)``."""
+        LongTensor [1, L_i], element i identical to ``sample(features[i:i+1], ...)``.
+        ``mode`` may also be a list / tuple of n_img style names: image i is captioned in style ``mode[i]`` (element i
+        identical to ``sample_batch(features[i:i+1], ..., mode=mode[i])[0]``), all styles in one beam search -- e.g.
+        ``sample_batch(feature.expand(4, -1), start, end, k, mode=list(STYLES))`` captions one image in every style."""
         from .decode import beam_sample
         return beam_sample(self, features, start_token, end_token, k, mode, feed_image)
 

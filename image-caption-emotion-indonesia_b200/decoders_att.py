@@ -610,12 +610,14 @@ class DecoderFactoredLSTMAtt(_AttBase):
 
     def sample(self, features, start_token, end_token, k=5, factual_limit=-1, mode="factual"):
         """Beam search with attention, stylenet/model_att.py:307-426."""
-        from .decode import beam_sample_att
+        from .decode import beam_sample_att, require_one_style
+        require_one_style(mode)
         return beam_sample_att(self, features, start_token, end_token, k, mode)[0]
 
     def sample_batch(self, features, start_token, end_token, k=5, mode="factual"):
         """``sample()`` for every image of ``features [n_img, S, S, D]`` in one batched beam search; returns a list of
-        LongTensor [1, L_i] (replaces the per-image loop of stylenet/evaluator.py:74-81)."""
+        LongTensor [1, L_i] (replaces the per-image loop of stylenet/evaluator.py:74-81).  ``mode`` may be a list /
+        tuple of n_img style names: image i in style ``mode[i]``, all in one beam search."""
         from .decode import beam_sample_att
         return beam_sample_att(self, features, start_token, end_token, k, mode)
 

@@ -1,7 +1,8 @@
 """Batched evaluation (SURVEY.md section 8 f2): the two loops that follow the decoder in the reference,
   * ``validate``  = val_factual / val_emotion of stylenet/train_multitask.py:272-361 (teacher_forcing_ratio = 0 forward,
     token loss, top-5 accuracy, per-caption arg-max ids for BLEU), and
-  * ``generate``  = the per-image ``sample()`` loop of stylenet/evaluator.py:63-101,
+  * ``generate``  = the per-image ``sample()`` loop of stylenet/evaluator.py:63-101 (``styles=``: every image in every
+    style, one mixed-style beam search per batch),
 with everything id-level done on the device: the loss / top-5 / arg-max come out of the fused softmax kernel instead of
 five passes over the [N, V] logits on the host, and beam search runs for a whole batch of images at once
 (``sample_batch``).  Corpus BLEU over the ids (``bleu.corpus_bleu``, nltk's semantics) runs on the device too:
@@ -69,11 +70,31 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
 
 
 @torch.no_grad()
-def generate(decoder, feature_batches, start_token, end_token, k=5, mode=None, encoder=None, **sample_kw):
+def generate(decoder, feature_batches, start_token, end_token, k=5, mode=None, encoder=None, styles=None, **sample_kw):
     """Beam-search captions for every image: ``feature_batches`` yields feature tensors ([n, E] / [n, S, S, D]) or, with
-    ``encoder``, image batches.  Returns a list of id lists (one per image, as ``sample()`` would return them)."""
+    ``encoder``, image batches.  Returns a list of id lists (one per image, as ``sample()`` would return them).
+    ``styles`` (style decoders, e.g. ``STYLES``): caption every image in every listed style with ONE mixed-style
+    ``sample_batch`` per feature batch; returns {style: [id lists]}, each entry equal to ``generate(..., mode=style)``."""
     decoder.eval()
     kw = dict(sample_kw)
+    if styles is not None:
+        styles = list(styles)
+        if mode is not None:
+            raise ValueError("generate() takes mode or styles, not both")
+        if not styles:
+            raise ValueError("empty styles")
+        if len(set(styles)) != len(styles):
+            raise ValueError("duplicate style in %r" % (styles,))
+        out = {s: [] for s in styles}
+        for x in feature_batches:
+            feats = encoder(x) if encoder is not None else x
+            n = feats.shape[0]
+            # image-major, style-minor: image i in style s is row i * len(styles) + s
+            rep = feats.repeat_interleave(len(styles), 0)
+            ids = decoder.sample_batch(rep, start_token, end_token, k=k, mode=styles * n, **kw)
+            for j, t in enumerate(ids):
+                out[styles[j % len(styles)]].append(t[0].tolist())
+        return out
     if mode is not None:
         kw["mode"] = mode
     out = []

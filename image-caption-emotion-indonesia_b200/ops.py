@@ -683,8 +683,12 @@ def bn1d_bwd(x, dy, gamma, save_mean, save_invstd, training, dx, dgamma, dbeta):
 SKINNY_MAX_ROWS = 16
 
 
+SKINNY_LINEAR_MAX_ROWS = 256       # sn_skinny_linear beyond 16 rows: chunks of <= 16 rows along grid.y
+
+
 def skinny_linear(W, X, out, R, bias=None, group_n=0, group_x=0, K=None, x_rows=None):
-    """out[:R] = X[:R] W^T + bias for R <= 16 rows; W [N, K] fp32 (row pitch W.stride(0)); grouped form see sn100.h.
+    """out[:R] = X[:R] W^T + bias for R <= SKINNY_LINEAR_MAX_ROWS rows (more than 16 in row chunks, each as a call on
+    its rows alone); W [N, K] fp32 (row pitch W.stride(0)); grouped form see sn100.h.
     ``x_rows`` (int32 [R]): gather the input rows, X[x_rows[r]] (embedding lookup folded into the stage)."""
     N = W.shape[0]
     K = K if K is not None else W.shape[1]
@@ -698,6 +702,20 @@ def decode_cell(cell, H, R, Wx, Kx, X, group_x, bx, Wh, bh, h_prev, c_prev, src_
                                _ptr(bx), _ptr(_req(Wh)), _ptr(bh), _ptr(_req(h_prev)), _ptr(_req(c_prev)),
                                _ptr(src_row), _ptr(x_rows), _ptr(_req(h_out)), _ptr(_req(c_out)), _stream()),
           "sn_decode_cell")
+
+
+def decode_cell_groups(cell, H, row_off, rows_max, Wx, Kx, X, group_x, bx, Wh, bh, h_prev, c_prev, src_row, h_out,
+                       c_out, x_rows=None):
+    """decode_cell for G = len(row_off) - 1 <= 4 row groups in one launch: group g (rows [row_off[g], row_off[g+1]),
+    ``row_off`` a device int32 tensor) uses Wx[g] / bx[g] of ``Wx`` [G, 4H, Kx] and ``bx`` [G, 4H]."""
+    G = row_off.numel() - 1
+    if Wx.dim() != 3 or Wx.shape[0] != G or bx.shape[0] != G:
+        raise ValueError("decode_cell_groups: Wx / bx need one leading entry per group (%d)" % G)
+    check(lib().sn_decode_cell_groups(cell, H, G, _ptr(_req(row_off, torch.int32)), int(rows_max), _ptr(_req(Wx)),
+                                      Wx.stride(1), Wx.stride(0), Kx, _ptr(_req(X)), X.stride(0), group_x, _ptr(_req(bx)),
+                                      bx.stride(0), _ptr(_req(Wh)), _ptr(bh), _ptr(_req(h_prev)), _ptr(_req(c_prev)),
+                                      _ptr(src_row), _ptr(x_rows), _ptr(_req(h_out)), _ptr(_req(c_out)), _stream()),
+          "sn_decode_cell_groups")
 
 
 def bleu_counts(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, max_sentence_len, max_group_tokens):

@@ -157,7 +157,8 @@ class DecoderFactoredLSTMStack(DecoderFactoredLSTM):
     def sample(self, features, start_token, end_token, k=5, factual_limit=-1, mode="factual", feed_image=False):
         """Beam search with the reference's semantics (stylenet/model.py:198-294) through the stack: every live beam
         carries one (h, c) per layer (oracle/stack.py::stack_sample)."""
-        from .decode import beam_sample
+        from .decode import beam_sample, require_one_style
+        require_one_style(mode)
         return beam_sample(self, features, start_token, end_token, k, mode, feed_image)[0]
 
 

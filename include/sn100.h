@@ -421,7 +421,16 @@ int32_t sn_split_limbs_rows(const float* src, int64_t G, int64_t K, int64_t C, i
  *   src_row (may be NULL) re-orders the incoming state per row (beam bookkeeping, model.py:275-279): h_out / c_out
  *   must not alias h_prev / c_prev.  x_rows (may be NULL): row r of the input is X[x_rows[r]] -- with the factored
  *   chain collapsed once per decode call (Wx = U_g S_g V_g, bx = U_g(S_g bV_g + bS_g) + bU_g) the embedding lookup,
- *   the three projection stages and the cell are this one kernel. */
+ *   the three projection stages and the cell are this one kernel.
+ *   sn_skinny_linear also takes more than sn_skinny_max_rows() rows (up to 256): balanced chunks of <= 16 rows along
+ *   grid.y, each chunk computed exactly as a call on those rows alone.
+ * sn_decode_cell_groups: sn_decode_cell for G <= 4 row groups in ONE launch -- the per-style sample() calls of one
+ *   image (app/backend/model.py's four get_sample calls per upload; forward_step, stylenet/model.py:115-155, with the
+ *   style's S in the chain) as one decode step.  Group g owns rows [row_off[g], row_off[g+1]) (row_off: device int32
+ *   [G+1], non-decreasing) and reads Wx + g*sWx, bx + g*sbx (the collapsed chain of its style); W_hh, b_hh, src_row,
+ *   x_rows and the state are shared over all rows, as in sn_decode_cell.  rows_max >= the largest group (host-known,
+ *   sizes the row chunks).  Each row's arithmetic is that of sn_decode_cell: a step of the mixed rows equals the
+ *   single-style step of the same rows bit for bit. */
 int32_t sn_skinny_max_rows(void);
 int32_t sn_skinny_linear(const float* W, int64_t ldw, int64_t N, int64_t K, const float* X, int64_t ldx,
                          int64_t R, int64_t group_n, int64_t group_x, const float* bias, float* out,
@@ -430,6 +439,11 @@ int32_t sn_decode_cell(int32_t cell, int64_t H, int64_t R, const float* Wx, int6
                        const float* X, int64_t ldx, int64_t group_x, const float* bx, const float* Wh,
                        const float* bh, const float* h_prev, const float* c_prev, const int32_t* src_row,
                        const int32_t* x_rows, float* h_out, float* c_out, void* stream);
+int32_t sn_decode_cell_groups(int32_t cell, int64_t H, int64_t G, const int32_t* row_off, int64_t rows_max,
+                              const float* Wx, int64_t ldwx, int64_t sWx, int64_t Kx, const float* X, int64_t ldx,
+                              int64_t group_x, const float* bx, int64_t sbx, const float* Wh, const float* bh,
+                              const float* h_prev, const float* c_prev, const int32_t* src_row, const int32_t* x_rows,
+                              float* h_out, float* c_out, void* stream);
 
 /* ---- encoder tail -> decoder hand-off (SURVEY.md section 8 f1) ---------------------------------------------------
  * sn_pool_nhwc_fwd: AdaptiveAvgPool2d((S,S)) + permute(0,2,3,1) of the trunk output (stylenet/model_att.py:24-28),
