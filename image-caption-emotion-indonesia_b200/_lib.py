@@ -33,6 +33,11 @@ SIGNATURES = {
     "sn_cast_bf16": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _P]),
     "sn_cast_bf16_ex": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _I32, _P]),
     "sn_colsum": (_I32, [_P, _I64, _I64, _I64, _P, _F, _P]),
+    "sn_colsum_ex": (_I32, [_P, _I64, _I64, _I64, _P, _F, _I32, _P]),
+    "sn_colsum_bf16_ex": (_I32, [_P, _I64, _I64, _I64, _P, _F, _I32, _P]),
+    "sn_embed_plan": (_I32, [_P, _I64, _I32, _P, _P, _P, _I64, _I64, _P, _P]),
+    "sn_embed_grad": (_I32, [_P, _I64, _P, _I64, _I32, _P, _P, _P, _I64, _P, _I64, _F, c_uint64, _P, _I64, _P, _P, _I32, _P]),
+    "sn_adam_clamp_dev_ex": (_I32, [_P, _P, _P, _P, _I32, _P, _P, _P, _P, _P, _F, _F, _F, _F, _I32, _P]),
     "sn_recur_ws_bytes": (_I64, [_I64, _I64]),
     "sn_recur_fwd": (_I32, [_I32, _I64, _I64, _P, _P, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "sn_recur_bwd": (_I32, [_I32, _I64, _I64, _P, _P, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -197,6 +197,55 @@ __global__ void embed_chunk_kernel(const int32_t* __restrict__ tok32, const int3
   }
 }
 
+// The same chunk sums as embed_chunk_kernel, bit for bit, with the latency of a chunk cut: one CTA per chunk and one
+// thread per column (blockDim.x >= E, a multiple of 32), the chunk's row ids and dropout rates staged in shared memory,
+// and the rows loaded EBW_BATCH at a time before they are added in row order.  A row with scale 0 is loaded but not
+// added, exactly as the warp kernel skips it (acc + 0 would turn an accumulated -0 into +0); the product-sum is the FFMA
+// the warp kernel compiles to.  The warp kernel pays one dependent load round per row: ~70 us at configs[1], where
+// the <start> token's 96 rows make three chunks of 32 (B200, profiles/README.md).
+constexpr int EBW_BATCH = 16;
+__global__ void __launch_bounds__(512) embed_chunk_wide_kernel(
+    const int32_t* __restrict__ tok32, const int32_t* __restrict__ start, const int32_t* __restrict__ cstart,
+    const int32_t* __restrict__ sorted, int64_t V, const int32_t* __restrict__ tok_override,
+    const float* __restrict__ dX, int64_t ldx, int E, float p, float inv_keep, uint64_t seed,
+    const uint64_t* __restrict__ seed_dev, float* __restrict__ dtable, float* __restrict__ part) {
+  __shared__ int32_t rows[EB_CHUNK];
+  __shared__ float rate[EB_CHUNK];
+  const int64_t i = blockIdx.x;
+  if (i >= start[V]) return;
+  const int32_t t = tok32[sorted[i]], s = start[t], e = start[t + 1];
+  if ((i - s) % EB_CHUNK) return;
+  if (seed_dev) seed += *seed_dev;
+  const int32_t n = (int32_t)(e - i < EB_CHUNK ? e - i : EB_CHUNK);
+  if (threadIdx.x < n) {
+    const int32_t j = sorted[i + threadIdx.x];
+    rows[threadIdx.x] = j;
+    rate[threadIdx.x] = (tok_override && tok_override[j] >= 0) ? 0.f : p;   // fed-back embeddings: no dropout
+  }
+  __syncthreads();
+  const int c = threadIdx.x;
+  if (c >= E) return;
+  float acc = 0.f;
+  for (int q0 = 0; q0 < n; q0 += EBW_BATCH) {
+    float x[EBW_BATCH], sc[EBW_BATCH];
+#pragma unroll
+    for (int u = 0; u < EBW_BATCH; ++u) {
+      const int q = q0 + u;
+      x[u] = 0.f; sc[u] = 0.f;
+      if (q < n) {
+        const int64_t j = rows[q];
+        x[u] = dX[j * ldx + c];
+        sc[u] = sn::dropout_scale(seed, (uint32_t)j, (uint32_t)c, rate[q], inv_keep);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < EBW_BATCH; ++u)
+      if (sc[u] != 0.f) acc = __fmaf_rn(x[u], sc[u], acc);
+  }
+  if (e - s <= EB_CHUNK) dtable[(int64_t)t * E + c] += acc;
+  else part[(int64_t)(cstart[t] + (i - s) / EB_CHUNK) * E + c] = acc;
+}
+
 // one warp per token whose group has several chunks: chunk sums in chunk order
 __global__ void embed_combine_kernel(const int32_t* __restrict__ cnt, const int32_t* __restrict__ cstart, int64_t V,
                                      int E, const float* __restrict__ part, float* __restrict__ dtable) {
@@ -776,29 +825,62 @@ int32_t sn_gather_pack_bwd(const int64_t* captions, int64_t cap_ld, float* dtabl
   SN_REQUIRE(N < (int64_t)1 << 30, "sn_gather_pack_bwd: N=%lld rows", (long long)N);
   if (N == 0) return 0;
   SN_REQUIRE(ws_int && ws_part, "sn_gather_pack_bwd: null work space");
+  if (int32_t rc = sn_embed_plan(captions, cap_ld, has_feat, row_b, row_t, tok_override, N, V, ws_int, stream)) return rc;
+  return sn_embed_grad(dtable, E, dfeatures, feat_ld, has_feat, row_b, row_t, tok_override, N, dX, ldx, p_drop, seed,
+                       seed_dev, V, ws_int, ws_part, 0, stream);
+}
+
+namespace {
+struct EmbedWs {      // layout of ws_int: see sn100.h
+  int32_t *cnt, *start, *cursor, *cstart, *tok32, *perm, *sorted;
+  EmbedWs(int32_t* ws, int64_t V, int64_t N)
+      : cnt(ws), start(cnt + V), cursor(start + V + 1), cstart(cursor + V), tok32(cstart + V), perm(tok32 + N),
+        sorted(perm + N) {}
+};
+}  // namespace
+
+int32_t sn_embed_plan(const int64_t* captions, int64_t cap_ld, int32_t has_feat, const int32_t* row_b,
+                      const int32_t* row_t, const int32_t* tok_override, int64_t N, int64_t V, int32_t* ws_int,
+                      void* stream) {
+  SN_REQUIRE(N >= 0 && N < (int64_t)1 << 30 && V > 0, "sn_embed_plan: bad dims N=%lld V=%lld", (long long)N, (long long)V);
+  if (N == 0) return 0;
+  SN_REQUIRE(ws_int, "sn_embed_plan: null work space");
+  cudaStream_t st = (cudaStream_t)stream;
+  EmbedWs w(ws_int, V, N);
+  SN_CUDA(cudaMemsetAsync(w.cnt, 0, sizeof(int32_t) * (size_t)V, st));
+  const unsigned g_rows = (unsigned)((N + 255) / 256);
+  embed_count_kernel<<<g_rows, 256, 0, st>>>(captions, cap_ld, has_feat, row_b, row_t, tok_override, N, w.tok32, w.cnt);
+  embed_scan_kernel<<<1, 1024, 0, st>>>(w.cnt, V, w.start, w.cursor, w.cstart);
+  embed_place_kernel<<<g_rows, 256, 0, st>>>(w.tok32, N, w.cursor, w.perm);
+  embed_order_kernel<<<g_rows, 256, 0, st>>>(w.tok32, w.start, w.perm, N, V, w.sorted);
+  return sn::check_launch("sn_embed_plan");
+}
+
+int32_t sn_embed_grad(float* dtable, int64_t E, float* dfeatures, int64_t feat_ld, int32_t has_feat,
+                      const int32_t* row_b, const int32_t* row_t, const int32_t* tok_override, int64_t N,
+                      const float* dX, int64_t ldx, float p_drop, uint64_t seed, const uint64_t* seed_dev, int64_t V,
+                      const int32_t* ws_int, float* ws_part, int32_t wide, void* stream) {
+  SN_REQUIRE(N >= 0 && N < (int64_t)1 << 30 && E > 0 && ldx >= E && V > 0, "sn_embed_grad: bad dims");
+  SN_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "sn_embed_grad: dropout p=%f out of [0,1)", p_drop);
+  if (N == 0) return 0;
+  SN_REQUIRE(ws_int && ws_part, "sn_embed_grad: null work space");
   cudaStream_t st = (cudaStream_t)stream;
   float inv_keep = 1.f / (1.f - p_drop);
   if (has_feat && dfeatures)
-    gather_pack_bwd_kernel<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(captions, cap_ld, dtable, (int)E, dfeatures,
+    gather_pack_bwd_kernel<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(nullptr, 0, dtable, (int)E, dfeatures,
                                                                      feat_ld, has_feat, row_b, row_t, tok_override, N,
                                                                      dX, ldx, p_drop, inv_keep, seed, seed_dev);
-  int32_t* cnt = ws_int;               // layout: see sn100.h
-  int32_t* start = cnt + V;
-  int32_t* cursor = start + V + 1;
-  int32_t* cstart = cursor + V;
-  int32_t* tok32 = cstart + V;
-  int32_t* perm = tok32 + N;
-  int32_t* sorted = perm + N;
-  SN_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)V, st));
-  const unsigned g_rows = (unsigned)((N + 255) / 256), g_warps = (unsigned)((N + 7) / 8);
-  embed_count_kernel<<<g_rows, 256, 0, st>>>(captions, cap_ld, has_feat, row_b, row_t, tok_override, N, tok32, cnt);
-  embed_scan_kernel<<<1, 1024, 0, st>>>(cnt, V, start, cursor, cstart);
-  embed_place_kernel<<<g_rows, 256, 0, st>>>(tok32, N, cursor, perm);
-  embed_order_kernel<<<g_rows, 256, 0, st>>>(tok32, start, perm, N, V, sorted);
-  embed_chunk_kernel<<<g_warps, 256, 0, st>>>(tok32, start, cstart, sorted, V, tok_override, dX, ldx, (int)E, p_drop,
-                                              inv_keep, seed, seed_dev, dtable, ws_part);
-  embed_combine_kernel<<<(unsigned)((V + 7) / 8), 256, 0, st>>>(cnt, cstart, V, (int)E, ws_part, dtable);
-  return sn::check_launch("sn_gather_pack_bwd");
+  EmbedWs w(const_cast<int32_t*>(ws_int), V, N);
+  if (wide && E <= 512)
+    embed_chunk_wide_kernel<<<(unsigned)N, (unsigned)((E + 31) / 32 * 32), 0, st>>>(
+        w.tok32, w.start, w.cstart, w.sorted, V, tok_override, dX, ldx, (int)E, p_drop, inv_keep, seed, seed_dev,
+        dtable, ws_part);
+  else
+    embed_chunk_kernel<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(w.tok32, w.start, w.cstart, w.sorted, V, tok_override,
+                                                                 dX, ldx, (int)E, p_drop, inv_keep, seed, seed_dev,
+                                                                 dtable, ws_part);
+  embed_combine_kernel<<<(unsigned)((V + 7) / 8), 256, 0, st>>>(w.cnt, w.cstart, V, (int)E, ws_part, dtable);
+  return sn::check_launch("sn_embed_grad");
 }
 
 int32_t sn_softmax_nll(const float* logits, int64_t N, int64_t V, int64_t ld, const int64_t* targets,
@@ -859,6 +941,14 @@ int32_t sn_adam_clamp(float* p, float* g, float* m, float* v, int32_t n_ranges, 
 int32_t sn_adam_clamp_dev(float* p, float* g, float* m, float* v, int32_t n_ranges, const int64_t* ranges,
                           const int32_t* step_idx, int32_t* steps_dev, const float* lr_dev, float* coef_ws,
                           float beta1, float beta2, float eps, float clip, void* stream) {
+  return sn_adam_clamp_dev_ex(p, g, m, v, n_ranges, ranges, step_idx, steps_dev, lr_dev, coef_ws, beta1, beta2, eps,
+                              clip, 0, stream);
+}
+
+int32_t sn_adam_clamp_dev_ex(float* p, float* g, float* m, float* v, int32_t n_ranges, const int64_t* ranges,
+                             const int32_t* step_idx, int32_t* steps_dev, const float* lr_dev, float* coef_ws,
+                             float beta1, float beta2, float eps, float clip, int32_t max_ctas, void* stream) {
+  SN_REQUIRE(max_ctas >= 0, "sn_adam_clamp_dev: max_ctas < 0");
   SN_REQUIRE(n_ranges >= 0 && n_ranges <= AdamRanges::MAX, "sn_adam_clamp_dev: at most %d ranges per call", AdamRanges::MAX);
   SN_REQUIRE(steps_dev && lr_dev && coef_ws, "sn_adam_clamp_dev: null argument");
   if (n_ranges == 0) return 0;
@@ -876,6 +966,7 @@ int32_t sn_adam_clamp_dev(float* p, float* g, float* m, float* v, int32_t n_rang
   int64_t chunks = R.chunk_start[R.n];
   if (chunks == 0) return sn::check_launch("sn_adam_clamp_dev");
   int64_t cap = (int64_t)sn::dev_info().sm_count * 8;
+  if (max_ctas > 0 && max_ctas < cap) cap = max_ctas;
   unsigned grid = (unsigned)(chunks < cap ? chunks : cap);
   adam_clamp_kernel<<<grid, 256, 0, st>>>(p, g, m, v, R, coef_ws, beta1, beta2, eps, clip);
   return sn::check_launch("sn_adam_clamp_dev");

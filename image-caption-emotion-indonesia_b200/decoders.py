@@ -103,7 +103,8 @@ class _DecoderBase(nn.Module):
     # pickled; the arena is rebuilt on first use).  The reference pickles the whole decoder every epoch
     # (save_checkpoint, stylenet/utils.py:62-90) and un-pickles it to resume (train_multitask.py:169-176).
     _TRANSIENT = ("_greedy_graphs", "_decode_sessions", "_side_streams", "_out_w16", "_out_w16_pref", "_out_w16_ev",
-                  "_out_h16", "_seed_dev", "_arena", "_att_cache", "_gate_flag", "_gate_armed", "_after_recur", "_bucket_hook")
+                  "_out_h16", "_seed_dev", "_arena", "_att_cache", "_gate_flag", "_gate_armed", "_after_recur", "_bucket_hook",
+                  "_emb_early")
 
     def __getstate__(self):
         st = self.__dict__.copy()
@@ -263,6 +264,22 @@ class _DecoderBase(nn.Module):
         c.tok_override = None
         if not all_tf:
             c.tok_override = torch.full((N,), -1, dtype=torch.int32, device=dev)
+        c.emb_ws = c.emb_ev = c.emb_zeroed = None
+        if self.__dict__.pop("_emb_early", False) and all_tf:
+            # the token grouping of the embedding backward needs only the captions and the plan, and nothing reads the
+            # embedding's gradient between the previous step's Adam and the backward's group sums: both run here, on
+            # a side stream next to the forward, instead of on the tail of the step
+            V = emb.weight.shape[0]
+            c.emb_ws = ops.embed_plan_ws(V, N, dev)      # allocated on the current stream, written on the side stream
+            c.emb_zeroed = a.gflat
+            gE = self._gview(a.gflat, [self._emb_name()], emb.weight.shape)
+            side = self._side(4)
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                ops.embed_plan(captions, has_feat, d["row_b"], d["row_t"], None, N, V, c.emb_ws)
+                gE.zero_()
+                c.emb_ev = torch.cuda.Event()
+                c.emb_ev.record(side)
         c.Ein = E
         c.w16 = {}      # bf16 weight shadows of this call (refreshed every forward)
         c.ev_early = c.ev_late = c.ev_first = None
@@ -425,7 +442,9 @@ class _DecoderBase(nn.Module):
             self._run_deferred()
             with torch.cuda.stream(self._fork()):
                 ops.gemm_bf16(ops.OP_TN, cl.dZb, cl.Hpb, 4 * H, H, N, 4 * H, H, C=gW, ldc=H)
-                ops.colsum(dZ, N, 4 * H, 4 * H, gbW)
+                ops.colsum(dZ, N, 4 * H, 4 * H, gbW, wide=bool(ops.TAIL_SCHEDULE[0]))
+            # d b_U (factored input projection) is the same column sum of dZ: copied from d b_hh on this side stream
+            cl.colsum_dZ = gbW if ops.TAIL_SCHEDULE[0] else None
             return self._input_projection_bwd(cl, dZ, gbuf)
         ops.recur_bwd(self.cell, H, B, d["bs"], d["off"], 0, T, Whh, None, cl.Call, cl.gates, dHall, dZ, dh, dc)
         # dW_hh = dZ^T Hprev ; d b_hh = colsum(dZ)
@@ -454,10 +473,18 @@ class _DecoderBase(nn.Module):
         emb = self._emb()
         E = emb.weight.shape[1]
         gE = self._gview(gbuf, [self._emb_name()], emb.weight.shape)
-        gE.zero_()
         dfeat = torch.empty(B, E, dtype=torch.float32, device=dev) if (need_dfeat and c.has_feat) else None
-        ops.gather_pack_bwd(c.captions, gE, dfeat, c.has_feat, d["row_b"], d["row_t"], c.tok_override, N, dX,
-                            c.p_drop, c.seed, seed_dev=c.seed_dev)
+        if getattr(c, "emb_ws", None) is not None:
+            # grouping and zeroing were issued by the forward (_run_forward): only the group sums are left
+            torch.cuda.current_stream().wait_event(c.emb_ev)
+            if gbuf is not c.emb_zeroed:
+                gE.zero_()
+            ops.embed_grad(gE, dfeat, c.has_feat, d["row_b"], d["row_t"], c.tok_override, N, dX, c.p_drop, c.seed,
+                           c.emb_ws, seed_dev=c.seed_dev, wide=True)
+        else:
+            gE.zero_()
+            ops.gather_pack_bwd(c.captions, gE, dfeat, c.has_feat, d["row_b"], d["row_t"], c.tok_override, N, dX,
+                                c.p_drop, c.seed, seed_dev=c.seed_dev)
         if dfeat is not None and c.feat_shape is not None:
             dfeat = dfeat.view(c.feat_shape)
         # the embedding is the last gradient of the step: its bucket starts right here, next to the W_hh / U and S / V
@@ -554,7 +581,7 @@ class _DecoderBase(nn.Module):
                             ops.gate_wait(gate)
                         ops.gemm_bf16(ops.OP_TN, dLb, Hb, V, H, N, dLb.stride(0), Hb.stride(0), C=gC, ldc=H,
                                       max_pairs=0 if mode_dc == 2 else ops.DC_MAX_PAIRS[0])
-                        ops.colsum_bf16(dLb, N, V, dLb.stride(0), gb)
+                        ops.colsum_bf16(dLb, N, V, dLb.stride(0), gb, wide=bool(ops.TAIL_SCHEDULE[0]))
                 if mode_dc == 0:
                     side_work()
                 else:
@@ -671,19 +698,23 @@ class _DecoderBase(nn.Module):
         return _HiddenFn.apply(anchor, features, self, plan, captions, coins, mode, save), plan
 
     def forward_loss(self, captions, lengths, features=None, targets=None, teacher_forcing_ratio=1.0,
-                     mode="factual", backward=True, n_global=None, grad_hook=None, early_step=None):
+                     mode="factual", backward=True, n_global=None, grad_hook=None, early_step=None, early_embed=False):
         """Fused training entry point (an addition beside the kept surface, SURVEY.md section 8b):
         forward -> mean token NLL -> (optionally) backward, with log-softmax/NLL/gradient fused in one
         pass over the logits and no autograd graph.  Populates ``.grad`` like ``loss.backward()`` after
         ``zero_grad()`` would.  Returns ``(loss[1], stats)`` with stats = dict(argmax, top5hit).
         ``n_global``: token count to normalise by (data parallel: the global count).
         ``early_step(names) -> bool``: called (bf16 mode, on side stream 0, right behind dC / db_C) when the gradients
-        of the vocabulary projection are final, so that the optimizer can update them under the reverse recurrence."""
+        of the vocabulary projection are final, so that the optimizer can update them under the reverse recurrence.
+        ``early_embed``: in a teacher-forced bf16 step, issue the embedding backward's token grouping and gradient
+        zeroing from the forward, on a side stream (the same results, off the tail of the step)."""
         self._check_inputs(captions, features)
         plan = get_plan(lengths)
         coins = self._coins(plan.T, teacher_forcing_ratio)
         captions = captions.contiguous()
         dev = captions.device
+        # (the gradient arena's embedding rows are zeroed early only when they hold no live gradient)
+        self.__dict__["_emb_early"] = bool(early_embed and backward and self.bf16 and self._emb().weight.grad is None)
         with torch.no_grad():
             c = self._run_forward(plan, captions, features, coins, mode, save=backward)
             N = plan.N
@@ -983,7 +1014,11 @@ class DecoderFactoredLSTM(_DecoderBase):
         sa.wait_stream(main)
         with torch.cuda.stream(sa):
             ops.gemm_bf16(ops.OP_TN, dZb, c.A2, H, F, N, 4 * H, 4 * F, C=gU, ldc=F, batch=4, sA=H, sB=F, sC=H * F)
-            ops.colsum(dZ, N, 4 * H, 4 * H, gbU)
+            wide = bool(ops.TAIL_SCHEDULE[0])
+            if getattr(c, "colsum_dZ", None) is not None:
+                gbU.copy_(c.colsum_dZ)          # written by _layer_bwd on this stream: the same sum, bit for bit
+            else:
+                ops.colsum(dZ, N, 4 * H, 4 * H, gbU, wide=wide)
             # stream 0 also carried dW_hh / db_hh of this layer (_layer_bwd): bucket {W_hh, U} is final here
             self._bucket_final([lp + pre + g + sfx for pre in ("W_", "U_") for g in GATES for sfx in (".weight", ".bias")])
         ops.gemm_bf16(ops.OP_NN, dZb, Ub, N, F, H, 4 * H, Fp, C=dA2, ldc=4 * F, Cb=dA2b, ldcb=4 * F, batch=4, sA=H,
@@ -991,13 +1026,13 @@ class DecoderFactoredLSTM(_DecoderBase):
         sb.wait_stream(main)
         with torch.cuda.stream(sb):
             ops.gemm_bf16(ops.OP_TN, dA2b, c.A1, F, F, N, 4 * F, 4 * F, C=gS, ldc=F, batch=4, sA=F, sB=F, sC=F * F)
-            ops.colsum(dA2, N, 4 * F, 4 * F, gbS)
+            ops.colsum(dA2, N, 4 * F, 4 * F, gbS, wide=wide)
         ops.gemm_bf16(ops.OP_NN, dA2b, Sb, N, F, F, 4 * F, Fp, C=dA1, ldc=4 * F, Cb=dA1b, ldcb=4 * F, batch=4, sA=F,
                       sB=F * Fp, sC=F, sCb=F)
         sb.wait_stream(main)
         with torch.cuda.stream(sb):
             ops.gemm_bf16(ops.OP_TN, dA1b, c.Xb, 4 * F, Ein, N, 4 * F, Ep, C=gV, ldc=Ein)
-            ops.colsum(dA1, N, 4 * F, 4 * F, gbV)
+            ops.colsum(dA1, N, 4 * F, 4 * F, gbV, wide=wide)
             self._bucket_final([lp + style_attr(c.mode, g) + sfx for g in GATES for sfx in (".weight", ".bias")] +
                                [lp + "V_" + g + sfx for g in GATES for sfx in (".weight", ".bias")])
         ops.gemm_bf16(ops.OP_NN, dA1b, Vb, N, Ein, 4 * F, 4 * F, Ep, C=dX, ldc=Ein)

@@ -14,6 +14,8 @@ import re
 import torch
 import torch.distributed as dist
 
+from . import ops
+
 
 def merged_ranges(arena, names, max_gap=64):
     """Flat (offset, length) ranges covering ``names`` in the arena, merged across alignment padding."""
@@ -109,6 +111,12 @@ BG_PUSH_SMS = [int(os.environ.get("SN_DP_BG_PUSH_SMS", "16"))]     # grid cap of
 BG_RECV_CTAS = [int(os.environ.get("SN_DP_BG_RECV_CTAS", "0"))]    # same for its receive side (512-thread CTAs)
 BG_WU = [os.environ.get("SN_DP_BG_WU", "0") == "1"]              # exchange the W_hh / U bucket in the background too
 PEER_BUCKETS = [False]           # also exchange the W_hh/U, S/V and embedding buckets as soon as they are final (slower: see step())
+
+
+def tail_schedule(world, bucketed):
+    """Whether a training step takes the tail schedule of ops.TAIL_SCHEDULE: single GPU, bucketed (bf16, no attention)
+    step, and the switch on.  The data-parallel exchange paths keep theirs."""
+    return bool(ops.TAIL_SCHEDULE[0]) and world == 1 and bool(bucketed)
 
 
 class DataParallelTrainer:
@@ -230,10 +238,16 @@ class DataParallelTrainer:
         if self.world == 1 and bucketed:
             # single GPU: Adam of each bucket runs on the side stream that produced it (under the reverse recurrence /
             # the projection backward); the rest follows at the end
+            tail = tail_schedule(self.world, bucketed)
+            emb = getattr(self.decoder, "_emb_name", lambda: None)()
+
             def early_step(names):
-                self.optimizer.step(only=names)
+                # the vocabulary, W_hh / U and S / V buckets run next to the dZ -> dA2 -> dA1 -> dX chain: their grid can
+                # be capped (ops.ADAM_BG_CTAS; full width measured fastest).  The embedding bucket ends the step: full width
+                cap = ops.ADAM_BG_CTAS[0] if (tail and list(names) != [emb]) else 0
+                self.optimizer.step(only=names, max_ctas=cap)
                 early.extend(names)
-            kw = dict(kw, early_step=early_step)
+            kw = dict(kw, early_step=early_step, early_embed=tail)
         loss, stats = self.forward_backward(captions, lengths, features, n_global=n_global, b_global=b_global,
                                             grad_hook=hook, **kw)
         if self.world > 1:

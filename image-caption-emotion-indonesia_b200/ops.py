@@ -167,10 +167,12 @@ def linear_nt(x, w, bias=None, out=None):
     return gemm(OP_NT, x, w, out, M, N, K, x.stride(0), w.stride(0), out.stride(0), bias=bias)
 
 
-def colsum(X, M, N, ldx, out, beta=0.0, x_off=0, out_off=0):
+def colsum(X, M, N, ldx, out, beta=0.0, x_off=0, out_off=0, wide=False):
+    """``wide``: 16-byte loads where X and ldx allow (the same bits as the scalar kernel)."""
     _req(X); _req(out)
-    check(lib().sn_colsum(ctypes.c_void_p(X.data_ptr() + 4 * x_off), M, N, ldx,
-                          ctypes.c_void_p(out.data_ptr() + 4 * out_off), float(beta), _stream()), "sn_colsum")
+    check(lib().sn_colsum_ex(ctypes.c_void_p(X.data_ptr() + 4 * x_off), M, N, ldx,
+                             ctypes.c_void_p(out.data_ptr() + 4 * out_off), float(beta), 1 if wide else 0, _stream()),
+          "sn_colsum")
     return out
 
 
@@ -192,9 +194,10 @@ def gather_pack_fwd(captions, table, features, has_feat, row_b, row_t, tok_overr
         Xb.stride(0) if Xb is not None else 0, _stream()), "sn_gather_pack_fwd")
 
 
-def colsum_bf16(X, M, N, ldx, out, beta=0.0):
+def colsum_bf16(X, M, N, ldx, out, beta=0.0, wide=False):
     _req(X, torch.bfloat16); _req(out)
-    check(lib().sn_colsum_bf16(_ptr(X), M, N, ldx, _ptr(out), float(beta), _stream()), "sn_colsum_bf16")
+    check(lib().sn_colsum_bf16_ex(_ptr(X), M, N, ldx, _ptr(out), float(beta), 1 if wide else 0, _stream()),
+          "sn_colsum_bf16")
     return out
 
 
@@ -214,6 +217,32 @@ def gather_pack_bwd(captions, dtable, dfeatures, has_feat, row_b, row_t, tok_ove
         N, _ptr(_req(dX)), dX.stride(0), float(p_drop), ctypes.c_uint64(seed), _ptr(seed_dev),
         V, _ptr(ws_int), _ptr(ws_part), _stream()),
           "sn_gather_pack_bwd")
+
+
+def embed_plan_ws(V, N, device):
+    """Work space of the token grouping of sn_embed_plan / sn_embed_grad (layout: include/sn100.h)."""
+    return torch.empty(4 * V + 1 + 3 * N, dtype=torch.int32, device=device)
+
+
+def embed_plan(captions, has_feat, row_b, row_t, tok_override, N, V, ws_int):
+    """Plan part of the embedding backward (sn_embed_plan): groups the token rows by token into ``ws_int``."""
+    cap = _req(captions, torch.int64)
+    check(lib().sn_embed_plan(_ptr(cap), cap.stride(0), 1 if has_feat else 0, _ptr(row_b), _ptr(row_t),
+                              _ptr(tok_override) if tok_override is not None else None, N, V, _ptr(_req(ws_int, torch.int32)),
+                              _stream()), "sn_embed_plan")
+
+
+def embed_grad(dtable, dfeatures, has_feat, row_b, row_t, tok_override, N, dX, p_drop, seed, ws_int, seed_dev=None,
+               wide=True):
+    """Gradient part (sn_embed_grad): group sums of dX into the zeroed ``dtable`` by the plan in ``ws_int``."""
+    V, E = dtable.shape
+    ws_part = torch.empty((N // 16 + 1) * E, dtype=torch.float32, device=dX.device)
+    check(lib().sn_embed_grad(
+        _ptr(_req(dtable)), E, _ptr(dfeatures) if dfeatures is not None else None,
+        dfeatures.stride(0) if dfeatures is not None else 0, 1 if has_feat else 0, _ptr(row_b), _ptr(row_t),
+        _ptr(tok_override) if tok_override is not None else None, N, _ptr(_req(dX)), dX.stride(0), float(p_drop),
+        ctypes.c_uint64(seed), _ptr(seed_dev), V, _ptr(_req(ws_int, torch.int32)), _ptr(ws_part), 1 if wide else 0, _stream()),
+          "sn_embed_grad")
 
 
 _ws_cache = {}
@@ -416,6 +445,16 @@ import os as _os
 DC_SCHEDULE = [int(_os.environ.get("SN_DC_SCHEDULE", "0"))]     # measured: 0 is the fastest (profiles/README.md, r2)
 DC_MAX_PAIRS = [int(_os.environ.get("SN_DC_MAX_PAIRS", "37"))]     # half of the 74 SM pairs (measured best, profiles/README.md r2)
 
+# schedule of the tail of a single-GPU bf16 training step (DESIGN.md section 4).  1 (default): the embedding's token
+# grouping and gradient zeroing run on a side stream at the start of a teacher-forced forward, the group sums use the
+# one-thread-per-column kernel, d b_hh / d b_U are one column sum plus a copy, and the column sums use 16-byte loads.
+# 0: the previous schedule.  Both compute the same bits.
+TAIL_SCHEDULE = [int(_os.environ.get("SN_TAIL_SCHEDULE", "1"))]
+# grid cap (CTAs of 256 threads) of the Adam buckets that run next to the projection-backward chain under the tail
+# schedule; 0 = full width.  Measured on a B200 at configs[1]: 74 CTAs 0.492 ms/step, 148 0.453, 296 0.426, full width
+# 0.421 (profiles/README.md, r4) -- a capped Adam only stretches out under the chain, so the default is no cap
+ADAM_BG_CTAS = [int(_os.environ.get("SN_ADAM_BG_CTAS", "0"))]
+
 # hold the side-stream work of the vocabulary backward behind sn_gate_wait (experiment, OFF: no gain on one GPU --
 # the step is bound by total work, not by the delayed clusters -- and a 2-GPU run with the peer exchange behind the
 # gate did not finish; profiles/README.md r2)
@@ -531,8 +570,9 @@ def recur_bwd_gemm(cell, H, B, plan, Whh_b, Call, gates, dHall, dZ, dZb, dc_carr
     LAUNCHES[0] += plan.T
 
 
-def adam_clamp_dev(p, g, m, v, ranges, step_idx, steps_dev, lr_dev, coef_ws, beta1, beta2, eps, clip):
-    """Clamp + Adam with step counters / learning rate in device memory (CUDA-graph replayable)."""
+def adam_clamp_dev(p, g, m, v, ranges, step_idx, steps_dev, lr_dev, coef_ws, beta1, beta2, eps, clip, max_ctas=0):
+    """Clamp + Adam with step counters / learning rate in device memory (CUDA-graph replayable).  ``max_ctas`` > 0 caps
+    the grid (a bucket updated next to the critical chain); it changes no result."""
     n = len(ranges)
     for i0 in range(0, n, 48):
         k = min(48, n - i0)
@@ -542,10 +582,10 @@ def adam_clamp_dev(p, g, m, v, ranges, step_idx, steps_dev, lr_dev, coef_ws, bet
             R[2 * i], R[2 * i + 1] = ranges[i0 + i]
             S[i] = step_idx[i0 + i]
         # (coefficient slots are indexed by step_idx: one work space serves every call, also concurrent ones)
-        check(lib().sn_adam_clamp_dev(_ptr(_req(p)), _ptr(_req(g)), _ptr(_req(m)), _ptr(_req(v)), k,
-                                      ctypes.cast(R, ctypes.c_void_p), ctypes.cast(S, ctypes.c_void_p),
-                                      _ptr(steps_dev), _ptr(lr_dev), _ptr(coef_ws), beta1, beta2, eps, clip,
-                                      _stream()), "sn_adam_clamp_dev")
+        check(lib().sn_adam_clamp_dev_ex(_ptr(_req(p)), _ptr(_req(g)), _ptr(_req(m)), _ptr(_req(v)), k,
+                                         ctypes.cast(R, ctypes.c_void_p), ctypes.cast(S, ctypes.c_void_p),
+                                         _ptr(steps_dev), _ptr(lr_dev), _ptr(coef_ws), beta1, beta2, eps, clip,
+                                         int(max_ctas), _stream()), "sn_adam_clamp_dev")
 
 
 def enable_peer_access(peer_device):

@@ -130,11 +130,12 @@ class FusedClampAdam:
 
     # -- step ------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def step(self, only=None, skip=None):
+    def step(self, only=None, skip=None, max_ctas=0):
         """``only`` / ``skip``: parameter names to restrict the step to / leave out.  A training step may update the
         vocabulary projection (43 % of the Adam traffic at configs[1]) on a side stream as soon as its gradient is
         final, under the reverse recurrence, and finish with ``step(skip=...)`` -- per-parameter step counters make
-        the two calls equivalent to one."""
+        the two calls equivalent to one.  ``max_ctas`` > 0 caps the grid of the arena ranges' kernel (a bucket updated
+        next to the critical chain); it changes no result."""
         a = self._state()
         self._sync_lr()
         items, foreign = a.grad_ranges()
@@ -151,7 +152,7 @@ class FusedClampAdam:
         idx = [self.index[name] for _, _, name in items]
         a.kernel_epoch += 1
         ops.adam_clamp_dev(a.flat, a.gflat, self.m, self.v, ranges, idx, self.steps_dev, self.lr_dev, self.coef_ws,
-                           b1, b2, self.eps, self.grad_clip)
+                           b1, b2, self.eps, self.grad_clip, max_ctas=max_ctas)
         # parameters outside the arena (foreign gradient tensors, extra params): same kernel, one range each
         for name in foreign:
             self._step_tensor(a.named[name], ("arena", name))

@@ -75,6 +75,18 @@ int32_t sn_gather_pack_bwd(const int64_t* captions, int64_t cap_ld, float* dtabl
                            const uint64_t* seed_dev, int64_t V, int32_t* ws_int, float* ws_part, void* stream);
 /* Deterministic: the token rows are grouped by token (V = rows of dtable) and summed in row order, without float
    atomics.  Work space: ws_int 4*V + 1 + 3*N int32, ws_part (N/16 + 1)*E floats. */
+/* sn_gather_pack_bwd in two parts.  The plan part groups the token rows by token: memset, count, scan, place and
+   order into ws_int.  It reads only the captions, the packing plan and tok_override, so it can run as soon as those
+   are final (in the forward, on a side stream).  The gradient part sums the groups from dX into dtable (zeroed by the
+   caller) and writes dfeatures.  plan + grad is exactly sn_gather_pack_bwd.  wide != 0 sums each chunk of a group
+   with one CTA of one thread per column (E <= 512; the same bits, a fraction of the latency). */
+int32_t sn_embed_plan(const int64_t* captions, int64_t cap_ld, int32_t has_feat, const int32_t* row_b,
+                      const int32_t* row_t, const int32_t* tok_override, int64_t N, int64_t V, int32_t* ws_int,
+                      void* stream);
+int32_t sn_embed_grad(float* dtable, int64_t E, float* dfeatures, int64_t feat_ld, int32_t has_feat,
+                      const int32_t* row_b, const int32_t* row_t, const int32_t* tok_override, int64_t N,
+                      const float* dX, int64_t ldx, float p_drop, uint64_t seed, const uint64_t* seed_dev, int64_t V,
+                      const int32_t* ws_int, float* ws_part, int32_t wide, void* stream);
 
 /* ---- K2: GEMM (all nn.Linear call sites: V_g/S_*_g/U_g model.py:119-150, C model.py:189-194,
  * encoder_att/decoder_att/f_beta/init_h/init_c model_att.py:59-61,192-193,283, LSTMCell's two
@@ -127,6 +139,12 @@ int32_t sn_colsum(const float* X, int64_t M, int64_t N, int64_t ldx, float* out,
                   void* stream);
 int32_t sn_colsum_bf16(const void* X, int64_t M, int64_t N, int64_t ldx, float* out, float beta,
                        void* stream);
+/* the same sums, bit for bit, with 16-byte loads (4 fp32 / 8 bf16 columns per thread) when wide != 0 and X and
+   ldx are 16-byte aligned; otherwise the scalar kernel */
+int32_t sn_colsum_ex(const float* X, int64_t M, int64_t N, int64_t ldx, float* out, float beta, int32_t wide,
+                     void* stream);
+int32_t sn_colsum_bf16_ex(const void* X, int64_t M, int64_t N, int64_t ldx, float* out, float beta, int32_t wide,
+                          void* stream);
 
 /* ---- K3: persistent recurrence (W_hh h + gates + cell), forward and reverse-time backward -----
  * replaces the hot loop stylenet/model.py:180-187 with forward_step's W_g(h_t)+sigmoid/tanh+cell
@@ -277,6 +295,12 @@ int32_t sn_adam_clamp_dev(float* p, float* g, float* m, float* v, int32_t n_rang
                           const int64_t* ranges, const int32_t* step_idx, int32_t* steps_dev,
                           const float* lr_dev, float* coef_ws, float beta1, float beta2, float eps,
                           float clip, void* stream);
+/* same, with the grid capped at max_ctas CTAs of 256 threads (0 = the full 8 per SM): buckets updated on a side stream
+   next to the critical chain leave it its SMs.  The grid size changes no element's result. */
+int32_t sn_adam_clamp_dev_ex(float* p, float* g, float* m, float* v, int32_t n_ranges,
+                             const int64_t* ranges, const int32_t* step_idx, int32_t* steps_dev,
+                             const float* lr_dev, float* coef_ws, float beta1, float beta2, float eps,
+                             float clip, int32_t max_ctas, void* stream);
 
 /* ---- K9: data-parallel exchange fused with the optimizer, over NVLink peer memory (no NCCL) ------------
  * The reference has no distributed code; this replaces what `ncclAllReduce` + K7 would do.  Every rank (one

@@ -23,11 +23,14 @@ with profile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
 ev = [e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA and "Memcpy" not in e.name and "Memset" not in e.name]
 ev.sort(key=lambda e: e.time_range.start)
 # split into replays by large gaps
+# (measured from the latest END so far: a short kernel that starts under a long one on another stream is no gap)
 groups, cur = [], [ev[0]]
-for a, b in zip(ev[:-1], ev[1:]):
-    if b.time_range.start - a.time_range.end > 100:  # us
+last_end = ev[0].time_range.end
+for b in ev[1:]:
+    if b.time_range.start - last_end > 100:  # us
         groups.append(cur); cur = []
     cur.append(b)
+    last_end = max(last_end, b.time_range.end)
 groups.append(cur)
 rep = groups[-1]
 t0 = rep[0].time_range.start
