@@ -13,7 +13,7 @@ from .dp import DataParallelTrainer, GradSync, merged_ranges  # noqa: F401
 from .graph import GraphedTrainStep  # noqa: F401
 from .stack import DecoderFactoredLSTMStack, MultitaskSchedule  # noqa: F401
 from .encoders import EncoderCNN, EncoderCNNAtt  # noqa: F401
-from . import bleu, checkpoint, evaluate, seq2seq  # noqa: F401
+from . import bleu, checkpoint, cider, evaluate, seq2seq  # noqa: F401
 
 try:  # attention variants
     from .decoders_att import DecoderFactoredLSTMAtt, DecoderRNNAtt  # noqa: F401

@@ -4,7 +4,7 @@ There is NO fallback: if the library is missing or the device is not sm_100 ever
 """
 import ctypes
 import os
-from ctypes import c_char_p, c_float, c_int32, c_int64, c_uint64, c_void_p
+from ctypes import c_char_p, c_double, c_float, c_int32, c_int64, c_uint64, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libsn100.so")
@@ -13,7 +13,7 @@ OP_NT, OP_NN, OP_TN = 0, 1, 2
 CELL_FACTORED, CELL_LSTM = 0, 1
 
 _P = c_void_p
-_I32, _I64, _F = c_int32, c_int64, c_float
+_I32, _I64, _F, _D = c_int32, c_int64, c_float, c_double
 
 # name -> (restype, argtypes); must list EVERY symbol include/sn100.h declares
 SIGNATURES = {
@@ -84,6 +84,8 @@ SIGNATURES = {
     "sn_bn1d_bwd": (_I32, [_P, _P, _I64, _I64, _P, _P, _P, _I32, _P, _P, _P, _P]),
     "sn_beam_step": (_I32, [_P, _I64, _I64, _I32, _I32, _I32, _I32, _I32] + [_P] * 15),
     "sn_bleu_counts": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _I64, _P, _P]),
+    "sn_cider_df": (_I32, [_P, _P, _P, _I64, _I32, _I32, _I64, _P, _P, _I64, _P, _P]),
+    "sn_cider_scores": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _D, _I32, _I64, _P, _P, _I64, _P, _P, _P]),
 }
 
 _lib = None

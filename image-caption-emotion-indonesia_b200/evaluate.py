@@ -5,12 +5,14 @@
     style, one mixed-style beam search per batch),
 with everything id-level done on the device: the loss / top-5 / arg-max come out of the fused softmax kernel instead of
 five passes over the [N, V] logits on the host, and beam search runs for a whole batch of images at once
-(``sample_batch``).  Corpus BLEU over the ids (``bleu.corpus_bleu``, nltk's semantics) runs on the device too:
-``validate(..., bleu_weights=...)`` adds it to the result, and ``generate``'s captions go to ``bleu.corpus_bleu`` once
-<start> / <end> are stripped.  Ids -> words stays with the caller."""
+(``sample_batch``).  Corpus BLEU over the ids (``bleu.corpus_bleu``, nltk's semantics) and CIDEr-D
+(``cider.corpus_cider``, coco-caption's semantics) run on the device too: ``validate(..., bleu_weights=..., cider=True)``
+adds them to the result, and ``generate``'s captions go to ``bleu.corpus_bleu`` / ``cider.CiderD`` once <start> / <end>
+are stripped.  Ids -> words stays with the caller."""
 import torch
 
 from .bleu import corpus_bleu
+from .cider import corpus_cider
 from .packing import get_plan
 
 
@@ -19,7 +21,8 @@ def _strip(ids, start, end):
 
 
 @torch.no_grad()
-def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, attention=None, bleu_weights=None):
+def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, attention=None, bleu_weights=None,
+             cider=False):
     """``batches`` yields (images_or_features, captions [B,T] int64, lengths, all_captions | None) like the reference's
     data loader (sorted by length, data_loader.py:116-145).  Returns dict(loss, top5 (percent), hypotheses,
     references, n_tokens) with the reference's definitions: loss = token-mean cross entropy averaged over batches
@@ -27,7 +30,8 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
     hypotheses = per-caption arg-max ids cut to the caption length with <start>/<end> removed.
     ``bleu_weights`` (a weight tuple or a list of them): the dict also holds "bleu" =
     ``bleu.corpus_bleu(references, hypotheses, bleu_weights)`` (train_multitask.py:341); every batch then needs its
-    all_captions, else ValueError."""
+    all_captions, else ValueError.  ``cider=True``: the dict also holds "cider" = the corpus CIDEr-D
+    ``cider.corpus_cider(references, hypotheses)[0]``, with the same need for all_captions."""
     was_training = decoder.training
     decoder.eval()
     if encoder is not None:
@@ -38,9 +42,9 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
     tot_tok = 0
     hyps, refs = [], []
     for images, captions, lengths, all_caps in batches:
-        if all_caps is None and bleu_weights is not None:
+        if all_caps is None and (bleu_weights is not None or cider):
             decoder.train(was_training)
-            raise ValueError("validate(bleu_weights=...) needs the references (all_captions) of every batch")
+            raise ValueError("validate(bleu_weights=... / cider=True) needs the references (all_captions) of every batch")
         feats = encoder(images) if encoder is not None else images
         lengths = [int(l) for l in lengths]
         if att:
@@ -66,6 +70,8 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
            "references": refs, "n_tokens": tot_tok}
     if bleu_weights is not None:
         res["bleu"] = corpus_bleu(refs, hyps, bleu_weights)
+    if cider:
+        res["cider"] = corpus_cider(refs, hyps)[0]
     return res
 
 

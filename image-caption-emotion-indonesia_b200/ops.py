@@ -771,6 +771,37 @@ def bleu_counts(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, max_sentence_len,
     return stats
 
 
+def cider_df(ref_tok, ref_off, ref_group, n, max_sentence_len, max_group_tokens, capacity, err):
+    """CIDEr-D document frequencies (sn_cider_df) of orders 1..n into a new table of ``capacity`` slots (a power of two):
+    returns (keys int32 [capacity, 4], counts int32 [capacity]), layout in include/sn100.h.  Inputs as for
+    ``bleu_counts`` without the hypotheses.  ``err`` (int32 CUDA tensor) receives the error bits; read it on the host
+    before trusting the table."""
+    dev = ref_group.device
+    keys = torch.empty(int(capacity), 4, dtype=torch.int32, device=dev)
+    counts = torch.empty(int(capacity), dtype=torch.int32, device=dev)
+    check(lib().sn_cider_df(_ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                            _ptr(_req(ref_group, torch.int64)), ref_group.numel() - 1, int(n), int(max_sentence_len),
+                            int(max_group_tokens), _ptr(keys), _ptr(counts), int(capacity),
+                            _ptr(_req(err, torch.int32)), _stream()), "sn_cider_df")
+    return keys, counts
+
+
+def cider_scores(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, n, sigma, max_sentence_len, max_group_tokens, keys,
+                 counts, out=None):
+    """CIDEr-D per image (sn_cider_scores) against the table of ``cider_df``: returns (scores float64 [n_img], per-order
+    sums float64 [n_img, 4]).  ``out``: a float64 [n_img] CUDA tensor to write the scores into."""
+    n_img = hyp_off.numel() - 1
+    scores = out if out is not None else torch.empty(n_img, dtype=torch.float64, device=hyp_off.device)
+    per_order = torch.empty(n_img, 4, dtype=torch.float64, device=hyp_off.device)
+    check(lib().sn_cider_scores(_ptr(_req(hyp_tok, torch.int32)), _ptr(_req(hyp_off, torch.int64)), n_img,
+                                _ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                                _ptr(_req(ref_group, torch.int64)), int(n), float(sigma), int(max_sentence_len),
+                                int(max_group_tokens), _ptr(_req(keys, torch.int32)), _ptr(_req(counts, torch.int32)),
+                                keys.shape[0], _ptr(_req(scores, torch.float64)), _ptr(per_order), _stream()),
+          "sn_cider_scores")
+    return scores, per_order
+
+
 def gate_wait(flag3, timeout_us=300):
     """Queue a one-thread kernel that returns once the cluster-form reverse recurrence (given the same flag) is resident."""
     check(lib().sn_gate_wait(_ptr(_req(flag3, torch.int32)), int(timeout_us), _stream()), "sn_gate_wait")

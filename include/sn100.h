@@ -511,6 +511,39 @@ int32_t sn_bleu_counts(const int32_t* hyp_tok, const int64_t* hyp_off, int64_t n
                        const int32_t* ref_tok, const int64_t* ref_off, const int64_t* ref_group,
                        int32_t max_sentence_len, int64_t max_group_tokens, int32_t* stats, void* stream);
 
+/* ---- K11: CIDEr-D (sn_cider.cu) -----------------------------------------------------------------------------------
+ * replaces coco-caption's CiderScorer (pycocoevalcap/cider/cider_scorer.py, Cider(n, sigma).compute_score) on integer
+ * token ids, document frequencies from the evaluated corpus.  Same CSR inputs as K10 (image i = hypothesis i and its
+ * references; sn_cider_df reads only the references), the same limits (max_sentence_len <= SN_BLEU_MAX_LEN, an
+ * image's tokens must fit in opt-in shared memory; either exceeded -> rc < 0 before any launch) and 1 <= n <= 4.
+ * Token ids must be non-negative: -1 pads the keys of the document-frequency table.
+ *
+ * sn_cider_df -- compute_doc_freq: counts[s] = number of images whose references contain the n-gram keys[s, :],
+ *   orders 1..n.  The table is caller memory: keys int32 [capacity, 4] (16-byte aligned; an n-gram of order k holds
+ *   its k ids followed by -1s, an empty slot is all -1), counts int32 [capacity], capacity a power of two (at least
+ *   2 x the number of reference n-grams keeps probe chains short).  The call clears the table and *err, then inserts
+ *   each n-gram of an image's references at its first occurrence across them (one int32 atomic add per image): the
+ *   counts are exact and independent of launch order.  Keys are compared in full; the hash only picks the first slot.
+ *   *err (device int32, read it after the stream): |1 the table is full (counts are then incomplete), |2 a negative
+ *   token id, |4 an image's sizes exceed the declared maxima.
+ * sn_cider_scores -- compute_cider: per image, in float64, with ref_len = log(n_img) and
+ *   idf(g) = ref_len - log(max(1, counts[g])) (an n-gram absent from the table has idf ref_len):
+ *   counts2vec  vec[g] = tf(g) * idf(g) over the distinct n-grams of a sentence, norm[k] = sqrt(sum vec^2 of order k),
+ *               length = number of bigrams (0 when n = 1: the scorer measures length on order index 1);
+ *   sim         val[k] = sum over hypothesis n-grams g of min(vec_h[g], vec_r[g]) * vec_r[g], divided by
+ *               norm_h[k] * norm_r[k] when both are non-zero, times e^(-(len_h - len_r)^2 / (2 sigma^2));
+ *   per_order[i, k] = sum of val[k] over the references of image i (k < n; 0 for k >= n; may be NULL),
+ *   scores[i]       = mean over the n orders of per_order[i, :] / (number of references) * 10.
+ *   Fixed summation order, no float atomics: run-to-run bitwise identical.  An image whose sizes exceed the declared
+ *   maxima gets NaN.  The corpus score is the mean of scores[]. */
+int32_t sn_cider_df(const int32_t* ref_tok, const int64_t* ref_off, const int64_t* ref_group, int64_t n_img,
+                    int32_t n, int32_t max_sentence_len, int64_t max_group_tokens, int32_t* keys, int32_t* counts,
+                    int64_t capacity, int32_t* err, void* stream);
+int32_t sn_cider_scores(const int32_t* hyp_tok, const int64_t* hyp_off, int64_t n_img, const int32_t* ref_tok,
+                        const int64_t* ref_off, const int64_t* ref_group, int32_t n, double sigma,
+                        int32_t max_sentence_len, int64_t max_group_tokens, const int32_t* keys,
+                        const int32_t* counts, int64_t capacity, double* scores, double* per_order, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
