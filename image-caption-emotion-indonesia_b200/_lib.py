@@ -29,7 +29,7 @@ SIGNATURES = {
     "sn_gemm2_bf16": (_I32, [_I32, _I64, _I64, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _I64, _P, _F, _I32, _I64, _I64, _I64, _I64, _I64, _I32, _P, _I64, _I32, _P]),
     "sn_vocab_ws_bytes": (_I64, [_I64, _I64]),
     "sn_vocab_nll_fwd": (_I32, [_I64, _I64, _I64, _P, _I64, _P, _I64, _P, _P, _P, _I64, _P, _P, _P, _P, _P, _P]),
-    "sn_vocab_nll_bwd": (_I32, [_I64, _I64, _I64, _P, _I64, _P, _I64, _P, _P, _P, _P, _F, _P, _I64, _P, _P, _P]),
+    "sn_vocab_nll_bwd": (_I32, [_I64, _I64, _I64, _P, _I64, _P, _I64, _P, _P, _P, _P, _F, _P, _P, _I64, _P, _P, _P]),
     "sn_cast_bf16": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _P]),
     "sn_cast_bf16_ex": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _I32, _P]),
     "sn_colsum": (_I32, [_P, _I64, _I64, _I64, _P, _F, _P]),
@@ -51,9 +51,9 @@ SIGNATURES = {
     "sn_recur_fwd_gemm": (_I32, [_I32, _I64, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "sn_recur_hprev": (_I32, [_P, _P, _P, _P, _I64, _I64, _P, _P]),
     "sn_recur_bwd_gemm": (_I32, [_I32, _I64, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
-    "sn_softmax_nll": (_I32, [_P, _I64, _I64, _I64, _P, _P, _P, _I64, _F, _P, _P, _P, _I64, _P]),
+    "sn_softmax_nll": (_I32, [_P, _I64, _I64, _I64, _P, _P, _P, _I64, _F, _P, _P, _P, _P, _I64, _P]),
     "sn_colsum_bf16": (_I32, [_P, _I64, _I64, _I64, _P, _F, _P]),
-    "sn_reduce_sum": (_I32, [_P, _I64, _F, _P, _I32, _P]),
+    "sn_reduce_sum": (_I32, [_P, _I64, _F, _P, _P, _I32, _P]),
     "sn_adam_clamp": (_I32, [_P, _P, _P, _P, _I32, _P, _P, _P, _F, _F, _F, _F, _P]),
     "sn_adam_clamp_dev": (_I32, [_P, _P, _P, _P, _I32, _P, _P, _P, _P, _P, _F, _F, _F, _F, _P]),
     "sn_enable_peer_access": (_I32, [_I32]),
@@ -86,6 +86,9 @@ SIGNATURES = {
     "sn_bleu_counts": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _I64, _P, _P]),
     "sn_cider_df": (_I32, [_P, _P, _P, _I64, _I32, _I32, _I64, _P, _P, _I64, _P, _P]),
     "sn_cider_scores": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _D, _I32, _I64, _P, _P, _I64, _P, _P, _P]),
+    "sn_cider_scores_rows": (_I32, [_P, _I64, _P, _I64, _I32, _P, _I64, _P, _P, _P, _I32, _D, _I32, _I64, _P, _P, _I64,
+                                    _P, _P]),
+    "sn_sample_step": (_I32, [_P, _I64, _I64, _I32, _I32, _I32, _D, _I32] + [_P] * 9),
 }
 
 _lib = None

@@ -133,3 +133,36 @@ class CiderD:
                                      max_group, self._keys, self._counts)
         scores = scores.cpu().numpy()
         return float(np.mean(scores)), scores
+
+    def score_samples(self, seqs, lengths, image_ids, start_token, end_token):
+        """CIDEr-D of sampled captions against this corpus, for self-critical training (scst.py): device float64 [R].
+        Row r's hypothesis is ``seqs[r, 1:lengths[r]]`` (column 0 holds ``start_token``) without a final
+        ``end_token`` -- the layout of ``sample_captions`` -- and its references are those of image ``image_ids[r]``
+        of the corpus this object was built from; idf uses that corpus' document frequencies and log(its image count),
+        not the number of rows.  ``seqs`` (int64 [R, ld]) and ``lengths`` (int64 [R]) stay on the device; ``image_ids``
+        is a host sequence of R corpus positions.  With ``image_ids = range(n_img)`` the scores equal those of
+        ``compute_score`` on the same hypotheses bit for bit.  Raises ValueError, before any device work, for a
+        ``seqs`` that is not 2-D, mismatched lengths and an image id out of range."""
+        if not isinstance(seqs, torch.Tensor) or seqs.dim() != 2:
+            raise ValueError("seqs must be a 2-D tensor [R, max_len]; got %s" % (
+                tuple(seqs.shape) if isinstance(seqs, torch.Tensor) else type(seqs).__name__,))
+        R, ld = seqs.shape
+        if not isinstance(lengths, torch.Tensor) or tuple(lengths.shape) != (R,):
+            raise ValueError("lengths must be a tensor of shape [%d]" % R)
+        ids = np.asarray(image_ids)
+        if ids.shape != (R,):
+            raise ValueError("%d image ids for %d rows" % (ids.size, R))
+        if R and (not np.issubdtype(ids.dtype, np.integer) or int(ids.min()) < 0 or int(ids.max()) >= self.n_img):
+            raise ValueError("image ids must be integers in 0..%d" % (self.n_img - 1))
+        ids = ids.astype(np.int64)
+        dev = self._ref_off.device
+        if R == 0:
+            return torch.empty(0, dtype=torch.float64, device=dev)
+        seqs = seqs.to(device=dev, dtype=torch.int64).contiguous()
+        lengths = lengths.to(device=dev, dtype=torch.int64).contiguous()
+        # shared-memory bounds from host-known sizes: the row width and the references of the images used
+        max_len = max(self._ref_max_len, ld - 1)
+        max_group = ld - 1 + int(self._ref_tokens[ids].max())
+        return ops.cider_scores_rows(seqs, lengths, torch.from_numpy(ids).to(dev), end_token, self.n_img, self._ref_tok,
+                                     self._ref_off, self._ref_group, self.n, self.sigma, max_len, max_group, self._keys,
+                                     self._counts)

@@ -151,10 +151,20 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
   return v;
 }
 
-// grid (n_img); block kScoreThreads; dynamic shared memory: kMaxOrder * max_len doubles (idf of the hypothesis
-// n-grams), kMaxOrder * max_len int32 (their tf, 0 where the n-gram is not a first occurrence), cap_tokens int32 ids
-__global__ void __launch_bounds__(kScoreThreads) cider_scores_kernel(
-    const int32_t* __restrict__ hyp_tok, const int64_t* __restrict__ hyp_off, const int32_t* __restrict__ ref_tok,
+// Where hypothesis i comes from.  CSR (kRows = false): hyp_tok[hyp_off[i] .. hyp_off[i + 1]), scored against image i.
+// Rows (kRows = true, sampled captions): seqs[i, 1 .. lengths[i]) without a final end_token, scored against image
+// img[i] of the corpus.
+struct HypRows {
+  const int64_t* seqs; int64_t ld; const int64_t* lengths; int32_t end_token; const int64_t* img;
+};
+
+// grid (number of hypotheses); block kScoreThreads; dynamic shared memory: kMaxOrder * max_len doubles (idf of the
+// hypothesis n-grams), kMaxOrder * max_len int32 (their tf, 0 where the n-gram is not a first occurrence), cap_tokens
+// int32 ids.  ref_len = log(n_corpus).
+template <bool kRows>
+__global__ void __launch_bounds__(kScoreThreads, kRows ? 1 : 0) cider_scores_kernel(
+    const int32_t* __restrict__ hyp_tok, const int64_t* __restrict__ hyp_off, HypRows rows, int64_t n_corpus,
+    const int32_t* __restrict__ ref_tok,
     const int64_t* __restrict__ ref_off, const int64_t* __restrict__ ref_group, int n, double sigma, int max_len,
     int64_t cap_tokens, const ulonglong2* __restrict__ keys, const int32_t* __restrict__ counts, uint64_t mask,
     double* __restrict__ scores, double* __restrict__ per_order) {
@@ -165,8 +175,17 @@ __global__ void __launch_bounds__(kScoreThreads) cider_scores_kernel(
   __shared__ double part_s[kScoreWarps][kMaxOrder];
   const int i = blockIdx.x;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t h0 = hyp_off[i], r0 = ref_group[i], r1 = ref_group[i + 1];
-  const int64_t L64 = hyp_off[i + 1] - h0;
+  int64_t h0, L64, gi = i;
+  if (kRows) {
+    h0 = (int64_t)i * rows.ld + 1;
+    L64 = rows.lengths[i] > rows.ld ? -1 : max((int64_t)0, rows.lengths[i] - 1);   // -1: past the row -> NaN below
+    if (L64 > 0 && rows.seqs[h0 + L64 - 1] == rows.end_token) --L64;
+    gi = rows.img[i];
+  } else {
+    h0 = hyp_off[i];
+    L64 = hyp_off[i + 1] - h0;
+  }
+  const int64_t r0 = ref_group[gi], r1 = ref_group[gi + 1];
   const int64_t base = ref_off[r0], nref_tok = ref_off[r1] - base;
   bool bad = L64 < 0 || L64 > max_len || nref_tok < 0 || L64 + nref_tok > cap_tokens;
   for (int64_t r = r0; r < r1 && !bad; ++r) bad = ref_off[r + 1] - ref_off[r] > max_len;
@@ -177,12 +196,12 @@ __global__ void __launch_bounds__(kScoreThreads) cider_scores_kernel(
   }
   const int L = (int)L64;
   const int nr = (int)nref_tok;
-  for (int t = threadIdx.x; t < L; t += kScoreThreads) tok[t] = hyp_tok[h0 + t];
+  for (int t = threadIdx.x; t < L; t += kScoreThreads) tok[t] = kRows ? (int32_t)rows.seqs[h0 + t] : hyp_tok[h0 + t];
   for (int t = threadIdx.x; t < nr; t += kScoreThreads) tok[L + t] = ref_tok[base + t];
   __syncthreads();
   const int32_t* hyp = tok;
   const int32_t* refs = tok + L;
-  const double ref_len = log((double)gridDim.x);
+  const double ref_len = log((double)n_corpus);
 
   // counts2vec of the hypothesis: tf and idf at the first occurrence of each n-gram, the squared norm per order
   double nh[kMaxOrder] = {0.0, 0.0, 0.0, 0.0};
@@ -325,9 +344,46 @@ extern "C" int32_t sn_cider_scores(const int32_t* hyp_tok, const int64_t* hyp_of
              "sn_cider_scores: a hypothesis and its references hold %lld tokens; at most %lld fit in shared memory",
              (long long)max_group_tokens, (long long)((optin - static_smem - hyp_bytes) / (int64_t)sizeof(int32_t)));
   if (smem > 48 * 1024)
-    SN_CUDA(cudaFuncSetAttribute(cider_scores_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  cider_scores_kernel<<<(unsigned)n_img, kScoreThreads, (size_t)smem, (cudaStream_t)stream>>>(
-      hyp_tok, hyp_off, ref_tok, ref_off, ref_group, n, sigma, max_sentence_len, max_group_tokens,
+    SN_CUDA(cudaFuncSetAttribute(cider_scores_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cider_scores_kernel<false><<<(unsigned)n_img, kScoreThreads, (size_t)smem, (cudaStream_t)stream>>>(
+      hyp_tok, hyp_off, HypRows{}, n_img, ref_tok, ref_off, ref_group, n, sigma, max_sentence_len, max_group_tokens,
       reinterpret_cast<const ulonglong2*>(keys), counts, (uint64_t)capacity - 1, scores, per_order);
   return sn::check_launch("cider_scores_kernel");
+}
+
+extern "C" int32_t sn_cider_scores_rows(const int64_t* seqs, int64_t ld, const int64_t* lengths, int64_t R,
+                                        int32_t end_token, const int64_t* img, int64_t n_corpus, const int32_t* ref_tok,
+                                        const int64_t* ref_off, const int64_t* ref_group, int32_t n, double sigma,
+                                        int32_t max_sentence_len, int64_t max_group_tokens, const int32_t* keys,
+                                        const int32_t* counts, int64_t capacity, double* scores, void* stream) {
+  SN_REQUIRE(R >= 0 && R <= 0x7fffffff, "sn_cider_scores_rows: R = %lld out of range", (long long)R);
+  SN_REQUIRE(n_corpus >= 1, "sn_cider_scores_rows: n_corpus = %lld", (long long)n_corpus);
+  SN_REQUIRE(ld >= 1 && ld - 1 <= max_sentence_len, "sn_cider_scores_rows: ld = %lld does not fit max_sentence_len = %d",
+             (long long)ld, (int)max_sentence_len);
+  SN_REQUIRE(max_group_tokens >= ld - 1, "sn_cider_scores_rows: max_group_tokens = %lld < ld - 1",
+             (long long)max_group_tokens);
+  SN_REQUIRE(n >= 1 && n <= kMaxOrder, "sn_cider_scores_rows: n = %d; orders 1..%d are supported", (int)n, kMaxOrder);
+  SN_REQUIRE(isfinite(sigma) && sigma > 0.0, "sn_cider_scores_rows: sigma = %g must be finite and > 0", sigma);
+  SN_REQUIRE(max_sentence_len >= 0 && max_sentence_len <= SN_BLEU_MAX_LEN,
+             "sn_cider_scores_rows: a sentence has %d tokens; the limit is %d", (int)max_sentence_len, SN_BLEU_MAX_LEN);
+  SN_REQUIRE(capacity > 0 && (capacity & (capacity - 1)) == 0,
+             "sn_cider_scores_rows: capacity = %lld is not a power of two", (long long)capacity);
+  if (R == 0) return 0;
+  SN_REQUIRE(seqs && lengths && img && ref_off && ref_group && keys && counts && scores,
+             "sn_cider_scores_rows: null argument");
+  SN_REQUIRE(((uintptr_t)keys & 15) == 0, "sn_cider_scores_rows: keys must be 16-byte aligned");
+  const int64_t hyp_bytes = (int64_t)kMaxOrder * max_sentence_len * (int64_t)(sizeof(double) + sizeof(int32_t));
+  const int64_t smem = hyp_bytes + max_group_tokens * (int64_t)sizeof(int32_t);
+  const int64_t static_smem = 2 * kScoreWarps * kMaxOrder * (int64_t)sizeof(double);
+  const int optin = sn::dev_info().smem_optin;
+  SN_REQUIRE(smem + static_smem <= optin,
+             "sn_cider_scores_rows: a hypothesis and its references hold %lld tokens; at most %lld fit in shared memory",
+             (long long)max_group_tokens, (long long)((optin - static_smem - hyp_bytes) / (int64_t)sizeof(int32_t)));
+  if (smem > 48 * 1024)
+    SN_CUDA(cudaFuncSetAttribute(cider_scores_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cider_scores_kernel<true><<<(unsigned)R, kScoreThreads, (size_t)smem, (cudaStream_t)stream>>>(
+      nullptr, nullptr, HypRows{seqs, ld, lengths, end_token, img}, n_corpus, ref_tok, ref_off, ref_group, n, sigma,
+      max_sentence_len, max_group_tokens, reinterpret_cast<const ulonglong2*>(keys), counts, (uint64_t)capacity - 1,
+      scores, nullptr);
+  return sn::check_launch("cider_scores_kernel(rows)");
 }

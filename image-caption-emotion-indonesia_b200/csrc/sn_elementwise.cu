@@ -268,7 +268,8 @@ __global__ void embed_combine_kernel(const int32_t* __restrict__ cnt, const int3
 __global__ void __launch_bounds__(256) softmax_nll_kernel(const float* __restrict__ logits, int64_t V, int64_t ld,
                                                           const int64_t* __restrict__ targets,
                                                           float* __restrict__ row_loss, float* dlogits, int64_t ldd,
-                                                          float grad_scale, int64_t* __restrict__ argmax,
+                                                          float grad_scale, const float* __restrict__ row_weight,
+                                                          int64_t* __restrict__ argmax,
                                                           int32_t* __restrict__ top5hit, int use_smem,
                                                           __nv_bfloat16* __restrict__ dlb, int64_t lddb) {
   extern __shared__ float srow[];
@@ -335,11 +336,12 @@ __global__ void __launch_bounds__(256) softmax_nll_kernel(const float* __restric
   __syncthreads();
   if (dlogits || dlb) {
     const float lse = bc_f[1];
+    const float gs = row_weight ? grad_scale * row_weight[row] : grad_scale;
     float* dst = dlogits ? dlogits + row * ldd : nullptr;
     __nv_bfloat16* dstb = dlb ? dlb + row * lddb : nullptr;
     for (int64_t c = tid; c < V; c += 256) {
       float pr = expf(rd[c] - lse);
-      float gr = (pr - (c == tgt ? 1.f : 0.f)) * grad_scale;
+      float gr = (pr - (c == tgt ? 1.f : 0.f)) * gs;
       if (dst) dst[c] = gr;
       if (dstb) dstb[c] = __float2bfloat16(gr);
     }
@@ -348,10 +350,13 @@ __global__ void __launch_bounds__(256) softmax_nll_kernel(const float* __restric
 }
 
 __global__ void __launch_bounds__(1024) reduce_sum_kernel(const float* __restrict__ x, int64_t N, float scale,
-                                                           float* out, int accumulate) {
+                                                           const float* __restrict__ w, float* out, int accumulate) {
   __shared__ double part[32];
   double s = 0.0;
-  for (int64_t i = threadIdx.x; i < N; i += 1024) s += (double)x[i];
+  if (w)
+    for (int64_t i = threadIdx.x; i < N; i += 1024) s += (double)x[i] * (double)w[i];
+  else
+    for (int64_t i = threadIdx.x; i < N; i += 1024) s += (double)x[i];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
@@ -884,8 +889,8 @@ int32_t sn_embed_grad(float* dtable, int64_t E, float* dfeatures, int64_t feat_l
 }
 
 int32_t sn_softmax_nll(const float* logits, int64_t N, int64_t V, int64_t ld, const int64_t* targets,
-                       float* row_loss, float* dlogits, int64_t ldd, float grad_scale, int64_t* argmax,
-                       int32_t* top5hit, void* dlogits_bf16, int64_t lddb, void* stream) {
+                       float* row_loss, float* dlogits, int64_t ldd, float grad_scale, const float* row_weight,
+                       int64_t* argmax, int32_t* top5hit, void* dlogits_bf16, int64_t lddb, void* stream) {
   SN_REQUIRE(N >= 0 && V > 0 && ld >= V, "sn_softmax_nll: bad dims");
   SN_REQUIRE(!dlogits_bf16 || lddb >= V, "sn_softmax_nll: lddb < V");
   if (N == 0) return 0;
@@ -899,14 +904,15 @@ int32_t sn_softmax_nll(const float* logits, int64_t N, int64_t V, int64_t ld, co
     }
   }
   softmax_nll_kernel<<<(unsigned)N, 256, use_smem ? smem : 0, (cudaStream_t)stream>>>(
-      logits, V, ld, targets, row_loss, dlogits, ldd, grad_scale, argmax, top5hit, use_smem,
+      logits, V, ld, targets, row_loss, dlogits, ldd, grad_scale, row_weight, argmax, top5hit, use_smem,
       (__nv_bfloat16*)dlogits_bf16, lddb);
   return sn::check_launch("sn_softmax_nll");
 }
 
-int32_t sn_reduce_sum(const float* x, int64_t N, float scale, float* out, int32_t accumulate, void* stream) {
+int32_t sn_reduce_sum(const float* x, int64_t N, float scale, const float* row_weight, float* out, int32_t accumulate,
+                      void* stream) {
   SN_REQUIRE(N >= 0 && out, "sn_reduce_sum: bad args");
-  reduce_sum_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(x, N, scale, out, accumulate);
+  reduce_sum_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(x, N, scale, row_weight, out, accumulate);
   return sn::check_launch("sn_reduce_sum");
 }
 

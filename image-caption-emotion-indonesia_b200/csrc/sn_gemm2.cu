@@ -63,7 +63,8 @@ struct Geo {
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_WARPS * XPOSE_BYTES + 1024 + 256;
 };
 
-enum { EPI_STORE = 0, EPI_PARTIAL = 1, EPI_STATS = 2, EPI_GRAD = 3, EPI_CELL_FWD = 4, EPI_CELL_BWD = 5 };
+enum { EPI_STORE = 0, EPI_PARTIAL = 1, EPI_STATS = 2, EPI_GRAD = 3, EPI_CELL_FWD = 4, EPI_CELL_BWD = 5,
+       EPI_GRADW = 6 /* EPI_GRAD with per-row weights */ };
 
 struct TmaSet { CUtensorMap m[4]; };
 
@@ -91,7 +92,11 @@ struct G2Args {
   float* h_out; __nv_bfloat16* hb_out; float* c_out; float* gates_out;
   const float* gates_in; const float* c_cur; const float* dh_in; float* dc_carry;   // bwd: [M,4H], [M,H], [M,H], [M,H]
   float* dz_out; __nv_bfloat16* dzb_out;                        // bwd: [M,4H] fp32 (optional) and bf16
+  const float* row_weight;         // EPI_GRADW: [M] per-row gradient weight
 };
+
+// EPI_GRADW: the one-hot term of a weighted row, |w| * scale
+__device__ __forceinline__ float wscale(const G2Args& g, int64_t row) { return fabsf(__ldg(g.row_weight + row)) * g.scale; }
 
 // ---- PTX wrappers ------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -754,9 +759,16 @@ gemm2_kernel(const __grid_constant__ TmaSet tma_a, const __grid_constant__ TmaSe
             }
           }
         }
-      } else {  // EPI_GRAD
+      } else {  // EPI_GRAD, EPI_GRADW
+        constexpr bool kW = EPI == EPI_GRADW;
         const int64_t tgt = row_ok ? g.targets[row] : -1;
-        const float escale = row_ok ? g.scale_log2 - g.lse[row] * LOG2E : 0.f;   // exp2 argument offset: -lse + log(scale)
+        // a row weight w scales the row's gradient: log2(|w| scale) joins the exponent offset, the one-hot term is
+        // |w| scale, and the sign is applied last (w = 0: exp2(-inf) = 0, so the row is zeros)
+        // (a separate instantiation, so the unweighted epilogue keeps its registers; the weighted one reads w (L1) where
+        // it is used instead of holding |w| scale and the sign across the loop, which spilled at the 96-register cap)
+        const float escale = row_ok ? (kW ? g.scale_log2 + log2f(fabsf(__ldg(g.row_weight + row))) : g.scale_log2) -
+                                          g.lse[row] * LOG2E
+                                    : 0.f;   // exp2 argument offset: -lse + log(scale); w = 1 adds an exact 0
         const float tl = row_ok ? g.tlogit[row] : 0.f;
         int cnt = 0;
 #pragma unroll 1
@@ -787,7 +799,7 @@ gemm2_kernel(const __grid_constant__ TmaSet tma_a, const __grid_constant__ TmaSe
             }
             if (tgt >= nb && tgt < nb + 32) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) if (nb + j == (int)tgt) v[j] -= g.scale;
+              for (int j = 0; j < 32; ++j) if (nb + j == (int)tgt) v[j] -= kW ? wscale(g, row) : g.scale;
             }
             if (!row_ok) {
               cnt = 0;
@@ -802,8 +814,13 @@ gemm2_kernel(const __grid_constant__ TmaSet tma_a, const __grid_constant__ TmaSe
               const bool in = row_ok && n < g.N;
               cnt += (in && x > tl);
               const float p = ex2(fmaf(x, LOG2E, escale));
-              v[j] = in ? p - (n == (int)tgt ? g.scale : 0.f) : 0.f;    // zeros = K padding of the next GEMMs
+              // zeros = K padding of the next GEMMs
+              v[j] = in ? p - (n == (int)tgt ? (kW ? wscale(g, row) : g.scale) : 0.f) : 0.f;
             }
+          }
+          if (kW && row_ok && __ldg(g.row_weight + row) < 0.f) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = -v[j];
           }
           if (g.dL) store_block_bf16(xbuf, lane, v, g.dL, g.lddl, row0, g.M, nb, (int)g.lddl, true);
         }
@@ -1055,8 +1072,8 @@ extern "C" int32_t sn_vocab_nll_fwd(int64_t N, int64_t V, int64_t H, const void*
 
 extern "C" int32_t sn_vocab_nll_bwd(int64_t N, int64_t V, int64_t H, const void* Hb, int64_t ldh, const void* Wb,
                                     int64_t ldw, const float* bias, const int64_t* targets, const float* tlogit,
-                                    const float* lse, float grad_scale, void* dL, int64_t lddl, int32_t* above,
-                                    int32_t* top5hit, void* stream) {
+                                    const float* lse, float grad_scale, const float* row_weight, void* dL,
+                                    int64_t lddl, int32_t* above, int32_t* top5hit, void* stream) {
   SN_REQUIRE(N >= 0 && V > 0 && H > 0, "sn_vocab_nll_bwd: bad dims");
   if (N == 0) return 0;
   SN_REQUIRE(bias && targets && tlogit && lse, "sn_vocab_nll_bwd: null argument");
@@ -1071,9 +1088,10 @@ extern "C" int32_t sn_vocab_nll_bwd(int64_t N, int64_t V, int64_t H, const void*
   rc = make_maps(SN_OP_NT, N, V, H, Hb, ldh, Wb, ldw, 1, 0, 0, ta, tb, g);
   if (rc) return rc;
   g.bias = bias; g.targets = targets; g.tlogit = (float*)tlogit; g.lse = lse; g.scale = grad_scale; g.scale_log2 = log2f(grad_scale);
+  g.row_weight = row_weight;
   g.dL = (__nv_bfloat16*)dL; g.lddl = dL ? lddl : V; g.above = above;
   cudaStream_t st = (cudaStream_t)stream;
-  rc = launch<EPI_GRAD>(ta, tb, g, st, "sn_vocab_nll_bwd");
+  rc = row_weight ? launch<EPI_GRADW>(ta, tb, g, st, "sn_vocab_nll_bwd") : launch<EPI_GRAD>(ta, tb, g, st, "sn_vocab_nll_bwd");
   if (rc) return rc;
   if (top5hit) {
     rank_hit_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(above, N, 5, top5hit);

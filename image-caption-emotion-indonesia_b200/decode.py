@@ -134,6 +134,8 @@ def _vocab_step(dec, h_new, logits, cache):
 
 
 class BeamState:
+    reorders = True          # the state rows follow the surviving beams (src_row) after every step
+
     def __init__(self, n_img, kmax, max_len, start_token, device):
         L = max_len + 2
         R = n_img * kmax
@@ -204,13 +206,58 @@ class BeamState:
         return [pk[i, :int(pk[i, L])].long().unsqueeze(0) for i in range(self.n_img)]
 
 
+class SampleState:
+    """Device state of a sampling decode (K12, ``sample_captions``): n independent samples of each of n_img images, row
+    i * n + j = sample j of image i.  No beam re-ordering: ``src_row`` is the identity.  ``seed_dev`` and ``step_dev``
+    feed the noise from device memory (include/sn100.h, sn_sample_step)."""
+    reorders = False
+
+    def __init__(self, n_img, n, max_len, start_token, temperature, greedy, device):
+        L = max_len + 2
+        R = n_img * n
+        self.n_img, self.kmax, self.max_len, self.L, self.R = n_img, n, max_len, L, R
+        self.start_token, self.temperature, self.greedy = start_token, float(temperature), bool(greedy)
+        i32 = dict(dtype=torch.int32, device=device)
+        self.prev_word = torch.full((R,), start_token, **i32)
+        self.src_row = torch.arange(R, **i32)
+        self.seqs = torch.zeros(R, L, dtype=torch.int64, device=device)
+        self.lengths = torch.zeros(R, dtype=torch.int64, device=device)
+        self.logprob = torch.zeros(R, L - 1, dtype=torch.float32, device=device)
+        self.done = torch.zeros(R, **i32)
+        self.n_unfinished = torch.full((1,), R, **i32)
+        self.step_dev = torch.ones(1, **i32)
+        self.seed_dev = torch.zeros(1, dtype=torch.int64, device=device)
+        self.reset()
+
+    def reset(self):
+        """Back to the state before the first draw (in place: the buffers may be baked into a CUDA graph)."""
+        self.prev_word.fill_(self.start_token)
+        self.seqs.zero_()
+        self.seqs[:, 0] = self.start_token
+        self.lengths.zero_()
+        self.logprob.zero_()
+        self.done.zero_()
+        self.n_unfinished.fill_(self.R)
+        self.step_dev.fill_(1)
+
+    def step(self, logits, step, end_token, device_step=False, advance=False):
+        """One draw per live row; the step index comes from ``step_dev``, which the caller advances (returns False)."""
+        ops.sample_step(logits, logits.shape[1], self.R, self.max_len, end_token, self.temperature, self.greedy,
+                        self.seed_dev, self.step_dev, self.prev_word, self.seqs, self.lengths, self.logprob, self.done,
+                        self.n_unfinished)
+        return False
+
+    def results(self):
+        return self.seqs.clone(), self.lengths.clone(), self.logprob.clone()
+
+
 class _DecodeSession:
     """Static buffers + (lazily captured) CUDA graphs of one decode step for a fixed (decoder, n_img, k, mode,
     start/end token).  ``sample()`` is called once per image by the reference's evaluation loops
     (stylenet/evaluator.py:74-81): replaying the captured step removes the ~12 Python-issued launches per step
     that otherwise make a single-image beam search launch-bound."""
 
-    def __init__(self, dec, n_img, k, mode, start_token, end_token):
+    def __init__(self, dec, n_img, k, mode, start_token, end_token, state=None):
         emb = dec._emb()
         dev = emb.weight.device
         E, H = emb.weight.shape[1], dec.hidden_size
@@ -218,7 +265,7 @@ class _DecodeSession:
         V = out.weight.shape[0]
         self._dec = weakref.ref(dec)          # the decoder owns its sessions: no reference cycle
         self.mode, self.end_token = mode, end_token
-        self.st = BeamState(n_img, k, dec.max_seq_length, start_token, dev)
+        self.st = state if state is not None else BeamState(n_img, k, dec.max_seq_length, start_token, dev)
         R = self.st.R
         f32 = dict(dtype=torch.float32, device=dev)
         self.L = L = _n_layers(dec)
@@ -259,7 +306,9 @@ class _DecodeSession:
             self.hB, self.cB = torch.zeros(L, R, H, **f32), torch.zeros(L, R, H, **f32)
             self.flip = 0              # 0: the state is in (h, c); 1: in (hB, cB)
 
-    def step(self, step, feed_image, device_step):
+    def step(self, step, feed_image, device_step, draw=True):
+        """One decode step.  ``draw=False``: advance the state only (the image step of sampling decode, whose output
+        is discarded)."""
         dec, st = self._dec(), self.st
         emb, out = dec._emb(), dec._out()
         R, H = st.R, dec.hidden_size
@@ -287,16 +336,21 @@ class _DecodeSession:
             ops.recur_fwd(dec.cell, H, R, self.bs1, self.off1, 0, 1, self.ctx.XP, Whh, bhh, self.h[l], self.h_new[l], None,
                           None, None, self.c[l])
             X = self.h_new[l]
-        _vocab_step(dec, self.h_new[self.L - 1], self.logits, self.cache)
-        st.step(self.logits, step, self.end_token, device_step=device_step)
-        idx = st.src_row.long()
-        for l in range(self.L):
-            torch.index_select(self.h_new[l], 0, idx, out=self.h[l])
-            c_new = self.c[l].index_select(0, idx)
-            self.c[l].copy_(c_new)
-        st.step_dev.add_(1)
+        if draw:
+            _vocab_step(dec, self.h_new[self.L - 1], self.logits, self.cache)
+            st.step(self.logits, step, self.end_token, device_step=device_step)
+        if st.reorders:
+            idx = st.src_row.long()
+            for l in range(self.L):
+                torch.index_select(self.h_new[l], 0, idx, out=self.h[l])
+                c_new = self.c[l].index_select(0, idx)
+                self.c[l].copy_(c_new)
+        else:
+            self.h.copy_(self.h_new)              # (recur_fwd updated c in place)
+        if draw:
+            st.step_dev.add_(1)
 
-    def step_skinny(self, step, feed_image, device_step):
+    def step_skinny(self, step, feed_image, device_step, draw=True):
         dec, st = self._dec(), self.st
         emb, out = dec._emb(), dec._out()
         R = st.R
@@ -327,16 +381,18 @@ class _DecodeSession:
                 kw["x_rows"] = rows
             dec._small_step(self.ctx, X, self.mode, R, src[0][l], src[1][l], st.src_row, dst[0][l], dst[1][l], **kw)
             X = dst[0][l]
-        ops.skinny_linear(out.weight, dst[0][self.L - 1], self.logits, R, bias=out.bias)
-        if not st.step(self.logits, step, self.end_token, device_step=device_step, advance=True):
-            st.step_dev.add_(1)
+        if draw:
+            ops.skinny_linear(out.weight, dst[0][self.L - 1], self.logits, R, bias=out.bias)
+            if not st.step(self.logits, step, self.end_token, device_step=device_step, advance=True):
+                st.step_dev.add_(1)
         self.flip ^= 1
 
     STEPS_PER_GRAPH = 4
 
     def capture_skinny(self):
-        """One graph = STEPS_PER_GRAPH consecutive steps (an even number: the state ends in the buffer it started in)."""
-        assert self.flip == 1 and self.STEPS_PER_GRAPH % 2 == 0
+        """One graph = STEPS_PER_GRAPH consecutive steps (an even number: the state ends in the buffer it started in).
+        Captured right after a restart: replays read the state from the buffer a restart leaves it in."""
+        assert self.STEPS_PER_GRAPH % 2 == 0
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
@@ -484,6 +540,100 @@ def beam_sample(dec, features, start_token, end_token, k, mode, feed_image, sync
             graph.replay()
         else:
             sess.step(step, feed_image, device_step=True)
+        if sync_every and step % sync_every == 0 and int(st.n_unfinished.item()) == 0:
+            break
+    return st.results()
+
+
+@torch.no_grad()
+def sample_decode(dec, features, start_token, end_token, n, mode, temperature, seed, greedy, sync_every=4):
+    """Sampling decode (``sample_captions``): n samples per row of ``features [n_img, E]`` on a ``_DecodeSession`` with a
+    ``SampleState``.  Step 0 feeds the image and discards its output, step 1 feeds <start>, step t the token drawn at
+    step t - 1 -- the conditioning of the teacher-forced ``forward_loss(captions, lengths, features)``.  Returns the
+    device tensors (seqs int64 [R, max_len + 2], lengths int64 [R], logprob float32 [R, max_len + 1])."""
+    emb = dec._emb()
+    E = emb.weight.shape[1]
+    dev = emb.weight.device
+    ops.lib()
+    dec.arena()
+    feats = features.detach().to(dev).float().reshape(-1, E)
+    n_img = feats.shape[0]
+    cache = dec.__dict__.setdefault("_decode_sessions", {})
+    key = ("sample", n_img, n, mode, start_token, end_token, dec.precision, float(temperature), bool(greedy))
+    sess = cache.get(key)
+    if sess is None or sess.arena_version != dec.arena().version:
+        if len(cache) > 8:
+            cache.clear()
+        st = SampleState(n_img, n, dec.max_seq_length, start_token, temperature, greedy, dev)
+        sess = cache[key] = _DecodeSession(dec, n_img, n, mode, start_token, end_token, state=st)
+    st = sess.st
+    sess.calls += 1
+    st.seed_dev.fill_(seed)
+    sess.feats.copy_(feats)
+    last = dec.max_seq_length + 1
+    if sess.skinny:
+        if COLLAPSE_CHAIN[0] and hasattr(dec, "_collapse_chain"):
+            for l in range(sess.L):
+                dec._collapse_chain(sess.ctx, mode, l)
+
+        def restart_eager():
+            st.reset()
+            sess.h.zero_()
+            sess.c.zero_()
+            sess.flip = 0
+            sess.step_skinny(1, True, True, draw=False)             # step 0: the image, output discarded
+            sess.step_skinny(1, False, True)                        # step 1: <start>, the first draw
+
+        def restart():
+            g0 = sess.__dict__.get("graph0_sample")
+            if g0 is None and sess.graph is not None:
+                s0 = torch.cuda.Stream()
+                s0.wait_stream(torch.cuda.current_stream())
+                with torch.cuda.stream(s0):
+                    restart_eager()
+                torch.cuda.current_stream().wait_stream(s0)
+                torch.cuda.synchronize()
+                g0 = torch.cuda.CUDAGraph()
+                with ops.no_gc_during_capture(), torch.cuda.graph(g0):
+                    restart_eager()
+                sess.graph0_sample = g0
+            if g0 is not None:
+                g0.replay()
+                sess.flip = 0
+            else:
+                restart_eager()
+        restart()
+        if sess.graph is None and sess.calls >= 2:
+            sess.capture_skinny()                                    # (runs throw-away steps: start over)
+            restart()
+        step = 2
+        while step <= last:
+            if sess.graph is not None:
+                sess.graph.replay()
+                step += sess.STEPS_PER_GRAPH
+            else:
+                for _ in range(sess.STEPS_PER_GRAPH):
+                    sess.step_skinny(step, False, device_step=True)
+                    step += 1
+            if int(st.n_unfinished.item()) == 0:
+                break
+        return st.results()
+    use_graph = not dec.bf16           # bf16 mode refreshes weight shadows per call: stays eager
+    if use_graph and sess.graph is None and sess.calls >= 2:
+        sess.capture()
+    st.reset()
+    sess.h.zero_()
+    sess.c.zero_()
+    sess.cache.clear()
+    sess.ctx.w16 = {}
+    sess.__dict__.pop("_w16_layers", None)
+    sess.step(1, True, True, draw=False)                             # step 0: the image, output discarded
+    graph = sess.graph if use_graph else None
+    for step in range(1, last + 1):
+        if graph is not None and step >= 2:
+            graph.replay()
+        else:
+            sess.step(step, False, device_step=True)
         if sync_every and step % sync_every == 0 and int(st.n_unfinished.item()) == 0:
             break
     return st.results()

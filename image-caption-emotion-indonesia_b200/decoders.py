@@ -595,13 +595,14 @@ class _DecoderBase(nn.Module):
         ops.colsum(dlogits, N, V, dlogits.stride(0), gb)
         return dHall
 
-    def _vocab_nll(self, Hall, Hb, targets, denom, backward):
+    def _vocab_nll(self, Hall, Hb, targets, denom, backward, row_weight=None):
         """Vocabulary projection + log-softmax + NLL (+ gradient w.r.t. the logits) + arg-max + top-5
         (stylenet/model.py:193-194, train_multitask.py:377-383, utils.py:127-140).
         bf16 mode: K5 fused with the projection -- logits live only in TMEM, never in HBM.  Pass 1 -> log-sum-exp,
         target logit, loss, arg-max; pass 2 recomputes the tiles and emits the gradient directly as the bf16
         operand of the dH / dC GEMMs (or only ranks the target when not training).
         fp32 mode: fp32 FFMA logits + the one-pass softmax kernel (gradient in place).
+        ``row_weight`` (float32 [N] or None): the gradient of row r is scaled by row_weight[r].
         Returns (row_loss, argmax, top5hit, dlogits_fp32 | None, dlogits_bf16 | None)."""
         out = self._out()
         V, H = out.weight.shape
@@ -623,12 +624,51 @@ class _DecoderBase(nn.Module):
             ops.vocab_nll_fwd(Hb, Wb, out.bias, targets, N, V, H, tl, lse, row_loss=row_loss, argmax=argmax, above=above)
             dLb = torch.empty(N, _pad8(V), dtype=torch.bfloat16, device=dev) if backward else None
             ops.vocab_nll_bwd(Hb, Wb, out.bias, targets, N, V, H, tl, lse, 1.0 / denom, dLb=dLb, above=above,
-                              top5hit=top5)
+                              top5hit=top5, row_weight=row_weight)
             return row_loss, argmax, top5, None, dLb
         logits = self._vocab_logits(Hall, Hb)
         ops.softmax_nll(logits, N, V, targets=targets, row_loss=row_loss, dlogits=logits if backward else None,
-                        grad_scale=1.0 / denom, argmax=argmax, top5hit=top5)
+                        grad_scale=1.0 / denom, argmax=argmax, top5hit=top5, row_weight=row_weight)
         return row_loss, argmax, top5, logits, None
+
+    # ---- sampling decode (self-critical training, scst.py) ----------------------------------------------------------
+    def sample_captions(self, features, start_token, end_token, n=1, temperature=1.0, seed=0, mode="factual",
+                        greedy=False):
+        """Draw ``n`` captions for each row of ``features [n_img, E]`` (K12, one pass over each step's logits with the
+        bookkeeping on the device; dropout off).  Returns device tensors
+          seqs     int64 [n_img * n, max_seq_length + 2], zero-padded; row i * n + j = sample j of image i,
+                   [<start>, w1, ..., <end>] (no <end> when the row ran out of steps);
+          lengths  int64 [n_img * n], counting <start> and <end>;
+          logprob  float32 [n_img * n, max_seq_length + 1]: column t - 1 = log-probability at temperature 1 of the
+                   token drawn at step t (zeros after the row's end).
+        Conditioning: step 0 feeds the image feature and discards its output, step 1 feeds <start>, step t the token
+        drawn at step t - 1; a row stops at its first <end> or after max_seq_length + 1 draws.  This is exactly the
+        teacher-forced ``forward_loss(seqs, lengths, features)``, so a sample is trained on as it is.  It is neither of
+        ``sample()``'s semantics: the reference's beam search never feeds the image, and ``feed_image=True`` (the app
+        back end) takes the first word from the image step.
+        Draw: token = argmax_v logit_v / temperature + g_v, Gumbel noise from a counter-based hash of (seed, step, row,
+        v) (include/sn100.h, sn_sample_step); ties to the lowest index.  ``greedy=True``: the plain arg-max.  The same
+        seed gives the same samples, eagerly or replayed from the session's CUDA graphs.
+        ``mode``: one style name (factored decoders; ignored by DecoderRNN).  Raises ValueError, before any device
+        work, for n < 1, a temperature that is not finite or not > 0, a seed outside 0 .. 2^63 - 1 and a style list."""
+        import math
+        import numbers
+        from .decode import sample_decode
+        if isinstance(n, bool) or not isinstance(n, numbers.Integral) or n < 1:
+            raise ValueError("n must be an integer >= 1; got %r" % (n,))
+        if not isinstance(temperature, numbers.Real) or not math.isfinite(temperature) or not temperature > 0:
+            raise ValueError("temperature must be finite and > 0; got %r" % (temperature,))
+        if isinstance(seed, bool) or not isinstance(seed, numbers.Integral) or not 0 <= seed < 1 << 63:
+            raise ValueError("seed must be an integer in 0 .. 2^63 - 1; got %r" % (seed,))
+        if isinstance(mode, (list, tuple)):
+            raise ValueError("sample_captions takes one style name, not a style list")
+        if self.cell == ops.CELL_FACTORED:
+            if mode not in STYLES:
+                raise ValueError("mode name wrong: %r (expected one of %s)" % (mode, STYLES))
+        else:
+            mode = None
+        return sample_decode(self, features, int(start_token), int(end_token), int(n), mode, float(temperature),
+                             int(seed), bool(greedy))
 
     # ---- greedy decoding (validation path) replayed from a CUDA graph ------------------------------------
     def _forward_greedy(self, captions, lengths, features, mode):
@@ -698,7 +738,8 @@ class _DecoderBase(nn.Module):
         return _HiddenFn.apply(anchor, features, self, plan, captions, coins, mode, save), plan
 
     def forward_loss(self, captions, lengths, features=None, targets=None, teacher_forcing_ratio=1.0,
-                     mode="factual", backward=True, n_global=None, grad_hook=None, early_step=None, early_embed=False):
+                     mode="factual", backward=True, n_global=None, grad_hook=None, early_step=None, early_embed=False,
+                     token_weights=None):
         """Fused training entry point (an addition beside the kept surface, SURVEY.md section 8b):
         forward -> mean token NLL -> (optionally) backward, with log-softmax/NLL/gradient fused in one
         pass over the logits and no autograd graph.  Populates ``.grad`` like ``loss.backward()`` after
@@ -707,9 +748,18 @@ class _DecoderBase(nn.Module):
         ``early_step(names) -> bool``: called (bf16 mode, on side stream 0, right behind dC / db_C) when the gradients
         of the vocabulary projection are final, so that the optimizer can update them under the reverse recurrence.
         ``early_embed``: in a teacher-forced bf16 step, issue the embedding backward's token grouping and gradient
-        zeroing from the forward, on a side stream (the same results, off the tail of the step)."""
+        zeroing from the forward, on a side stream (the same results, off the tail of the step).
+        ``token_weights``: float32 CUDA tensor [N] in packed row order (or None): the loss becomes
+        sum_r w_r * NLL_r / denom and every gradient is that loss's (weights may be negative, e.g. the advantages of
+        self-critical training, scst.py).  ``stats["argmax"]`` / ``"top5hit"`` and the per-row NLL do not depend on
+        it; weights of 1 give the unweighted results bit for bit."""
         self._check_inputs(captions, features)
         plan = get_plan(lengths)
+        if token_weights is not None:
+            if (not isinstance(token_weights, torch.Tensor) or token_weights.dtype != torch.float32
+                    or tuple(token_weights.shape) != (plan.N,) or token_weights.device != captions.device):
+                raise ValueError("token_weights must be a float32 tensor of shape [%d] on %s" % (plan.N, captions.device))
+            token_weights = token_weights.contiguous()
         coins = self._coins(plan.T, teacher_forcing_ratio)
         captions = captions.contiguous()
         dev = captions.device
@@ -737,10 +787,11 @@ class _DecoderBase(nn.Module):
                 else:
                     targets = self._default_targets(captions, plan, True)
             denom = float(n_global if n_global is not None else N)
-            row_loss, argmax, top5, logits, dLb = self._vocab_nll(c.top.Hall, c.top.Hb, targets, denom, backward)
+            row_loss, argmax, top5, logits, dLb = self._vocab_nll(c.top.Hall, c.top.Hb, targets, denom, backward,
+                                                                  row_weight=token_weights)
             loss = torch.empty(1, dtype=torch.float32, device=dev)
             if not (backward and dLb is not None):
-                ops.reduce_sum(row_loss, N, 1.0 / denom, loss)
+                ops.reduce_sum(row_loss, N, 1.0 / denom, loss, row_weight=token_weights)
             if backward:
                 gbuf = self._grad_target(c.grad_names + list(self._out_names()))
                 deferred = []
@@ -750,7 +801,7 @@ class _DecoderBase(nn.Module):
                     def loss_and_bucket():
                         # the scalar loss is bookkeeping: reduce it behind dC on side stream 0, not in front of dH
                         with torch.cuda.stream(self._side(0)):
-                            ops.reduce_sum(row_loss, N, 1.0 / denom, loss)
+                            ops.reduce_sum(row_loss, N, 1.0 / denom, loss, row_weight=token_weights)
                             if early_step is not None and gbuf is self.arena().gflat:
                                 self._publish(list(self._out_names()), gbuf)
                                 early_step(list(self._out_names()))

@@ -273,18 +273,20 @@ def recur_bwd(cell, H, B, bs, off, t0, t1, Whh, c_init, Call, gates, dHall, dZ, 
 
 
 def softmax_nll(logits, N, V, targets=None, row_loss=None, dlogits=None, grad_scale=1.0, argmax=None,
-                top5hit=None, row_off=0, dlogits_bf16=None):
+                top5hit=None, row_off=0, dlogits_bf16=None, row_weight=None):
     ld = logits.stride(0)
     check(lib().sn_softmax_nll(
         ctypes.c_void_p(logits.data_ptr() + 4 * row_off * ld), N, V, ld, _ptr(targets), _ptr(row_loss),
-        _ptr(dlogits), dlogits.stride(0) if dlogits is not None else 0, float(grad_scale), _ptr(argmax),
+        _ptr(dlogits), dlogits.stride(0) if dlogits is not None else 0, float(grad_scale),
+        _ptr(None if row_weight is None else _req(row_weight)), _ptr(argmax),
         _ptr(top5hit), _ptr(dlogits_bf16), dlogits_bf16.stride(0) if dlogits_bf16 is not None else 0,
         _stream()), "sn_softmax_nll")
 
 
-def reduce_sum(x, N, scale, out, accumulate=False):
-    check(lib().sn_reduce_sum(_ptr(_req(x)), N, float(scale), _ptr(out), 1 if accumulate else 0, _stream()),
-          "sn_reduce_sum")
+def reduce_sum(x, N, scale, out, accumulate=False, row_weight=None):
+    """out = scale * sum(x[:N] * row_weight[:N]) (row_weight None: weight 1)."""
+    check(lib().sn_reduce_sum(_ptr(_req(x)), N, float(scale), _ptr(None if row_weight is None else _req(row_weight)),
+                              _ptr(out), 1 if accumulate else 0, _stream()), "sn_reduce_sum")
 
 
 def adam_clamp(p, g, m, v, ranges, step_sizes, bc2_sqrts, beta1, beta2, eps, clip):
@@ -412,11 +414,14 @@ def vocab_nll_fwd(Hb, Wb, bias, targets, N, V, H, tlogit, lse, row_loss=None, ar
     LAUNCHES[0] += 1
 
 
-def vocab_nll_bwd(Hb, Wb, bias, targets, N, V, H, tlogit, lse, grad_scale, dLb=None, above=None, top5hit=None):
-    """Recompute the logits tiles; write (softmax - onehot) * grad_scale as bf16 [N, ld]; rank of the target."""
+def vocab_nll_bwd(Hb, Wb, bias, targets, N, V, H, tlogit, lse, grad_scale, dLb=None, above=None, top5hit=None,
+                  row_weight=None):
+    """Recompute the logits tiles; write (softmax - onehot) * grad_scale (* row_weight[row]) as bf16 [N, ld]; rank of
+    the target."""
     _req(Hb, torch.bfloat16); _req(Wb, torch.bfloat16); _req(targets, torch.int64)
     check(lib().sn_vocab_nll_bwd(N, V, H, _ptr(Hb), Hb.stride(0), _ptr(Wb), Wb.stride(0), _ptr(_req(bias)),
-                                 _ptr(targets), _ptr(tlogit), _ptr(lse), float(grad_scale), _ptr(dLb),
+                                 _ptr(targets), _ptr(tlogit), _ptr(lse), float(grad_scale),
+                                 _ptr(None if row_weight is None else _req(row_weight)), _ptr(dLb),
                                  dLb.stride(0) if dLb is not None else 0, _ptr(above), _ptr(top5hit), _stream()),
           "sn_vocab_nll_bwd")
     if top5hit is not None:
@@ -800,6 +805,35 @@ def cider_scores(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, n, sigma, max_se
                                 keys.shape[0], _ptr(_req(scores, torch.float64)), _ptr(per_order), _stream()),
           "sn_cider_scores")
     return scores, per_order
+
+
+def cider_scores_rows(seqs, lengths, img, end_token, n_corpus, ref_tok, ref_off, ref_group, n, sigma, max_sentence_len,
+                      max_group_tokens, keys, counts):
+    """CIDEr-D of sampled captions (sn_cider_scores_rows): row r = seqs[r, 1:lengths[r]] without a final end_token,
+    against the references of corpus image img[r], idf from the table of ``cider_df`` and log(n_corpus).  Returns
+    float64 [R]."""
+    R = seqs.shape[0]
+    scores = torch.empty(R, dtype=torch.float64, device=seqs.device)
+    check(lib().sn_cider_scores_rows(_ptr(_req(seqs, torch.int64)), seqs.stride(0), _ptr(_req(lengths, torch.int64)), R,
+                                     int(end_token), _ptr(_req(img, torch.int64)), int(n_corpus),
+                                     _ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                                     _ptr(_req(ref_group, torch.int64)), int(n), float(sigma), int(max_sentence_len),
+                                     int(max_group_tokens), _ptr(_req(keys, torch.int32)),
+                                     _ptr(_req(counts, torch.int32)), keys.shape[0], _ptr(scores), _stream()),
+          "sn_cider_scores_rows")
+    return scores
+
+
+def sample_step(logits, V, R, max_len, end_token, temperature, greedy, seed_dev, step_dev, prev_word, seqs, lengths,
+                logprob, done, n_unfinished):
+    """K12: one sampling-decode draw per live row of ``logits`` (Gumbel-max at ``temperature``, or the arg-max), with
+    the row bookkeeping on the device (include/sn100.h)."""
+    check(lib().sn_sample_step(_ptr(_req(logits)), logits.stride(0), V, R, max_len, int(end_token), float(temperature),
+                               1 if greedy else 0, _ptr(_req(seed_dev, torch.int64)), _ptr(_req(step_dev, torch.int32)),
+                               _ptr(_req(prev_word, torch.int32)), _ptr(_req(seqs, torch.int64)),
+                               _ptr(_req(lengths, torch.int64)), _ptr(_req(logprob)), _ptr(_req(done, torch.int32)),
+                               _ptr(_req(n_unfinished, torch.int32)), _stream()), "sn_sample_step")
+    LAUNCHES[0] += 1
 
 
 def gate_wait(flag3, timeout_us=300):

@@ -250,9 +250,12 @@ int32_t sn_recur_bwd_gemm(int32_t cell, int64_t H, int64_t B, const int32_t* bs_
  * row_loss[N] = lse - logit[target]; dlogits = (softmax - onehot) * grad_scale (may alias logits, may
  * be NULL); argmax[N] lowest index on ties (torch.max); top5hit[N] = 1 if fewer than 5 logits exceed
  * the target's.  targets may be NULL (then only argmax is produced).  dlogits_bf16 (optional, [N,lddb],
- * columns V..lddb zero): the gradient as the bf16 operand of the two vocab-projection backward GEMMs. */
+ * columns V..lddb zero): the gradient as the bf16 operand of the two vocab-projection backward GEMMs.
+ * row_weight (optional, float [N], any sign): the gradient of row r is multiplied by row_weight[r] (the gradient of
+ * sum_r w_r * row_loss_r * grad_scale); row_loss, argmax and top5hit do not depend on it.  NULL = weight 1, with the
+ * arithmetic of a call without weights. */
 int32_t sn_softmax_nll(const float* logits, int64_t N, int64_t V, int64_t ld, const int64_t* targets,
-                       float* row_loss, float* dlogits, int64_t ldd, float grad_scale,
+                       float* row_loss, float* dlogits, int64_t ldd, float grad_scale, const float* row_weight,
                        int64_t* argmax, int32_t* top5hit, void* dlogits_bf16, int64_t lddb, void* stream);
 /* K5 fused with the vocabulary projection (bf16 mode): logits = Hb Wb^T + bias are produced tile by tile in
  * TMEM and consumed by the epilogue -- the [N,V] logits are NEVER written to HBM.
@@ -263,6 +266,9 @@ int32_t sn_softmax_nll(const float* logits, int64_t N, int64_t V, int64_t ld, co
  * sn_vocab_nll_bwd: recomputes the logits tiles and writes dL = (softmax - onehot) * grad_scale as the bf16
  *   [N, lddl] operand of the two backward GEMMs (columns V..lddl zero; dL may be NULL = ranking only);
  *   above[row] += #{v : logit_v > logit_target}; top5hit[row] = above[row] < 5 (optional).
+ *   row_weight (optional, float [N], any sign): dL of row r = (softmax - onehot) * grad_scale * row_weight[r], with
+ *   log2(|w| * grad_scale) folded into the exponent offset and the sign applied after it (w = 0 writes zeros); NULL =
+ *   the arithmetic of a call without weights.
  * Hb [N,ldh], Wb [V,ldw]: bf16, K = H padded per the TMA rules of sn_gemm_bf16. */
 int64_t sn_vocab_ws_bytes(int64_t N, int64_t V);
 int32_t sn_vocab_nll_fwd(int64_t N, int64_t V, int64_t H, const void* Hb, int64_t ldh, const void* Wb,
@@ -271,11 +277,12 @@ int32_t sn_vocab_nll_fwd(int64_t N, int64_t V, int64_t H, const void* Hb, int64_
                          void* stream);
 int32_t sn_vocab_nll_bwd(int64_t N, int64_t V, int64_t H, const void* Hb, int64_t ldh, const void* Wb,
                          int64_t ldw, const float* bias, const int64_t* targets, const float* tlogit,
-                         const float* lse, float grad_scale, void* dL, int64_t lddl, int32_t* above,
-                         int32_t* top5hit, void* stream);
-/* loss = scale * sum(row_loss[0..N)) (+ loss if accumulate), deterministic order, double sum */
-int32_t sn_reduce_sum(const float* x, int64_t N, float scale, float* out, int32_t accumulate,
-                      void* stream);
+                         const float* lse, float grad_scale, const float* row_weight, void* dL, int64_t lddl,
+                         int32_t* above, int32_t* top5hit, void* stream);
+/* loss = scale * sum(row_loss[0..N) * row_weight[0..N)) (+ loss if accumulate), deterministic order, double sum;
+ * row_weight may be NULL (weight 1, the products are skipped) */
+int32_t sn_reduce_sum(const float* x, int64_t N, float scale, const float* row_weight, float* out,
+                      int32_t accumulate, void* stream);
 
 /* ---- K7: fused clamp + Adam over flat parameter ranges ---------------------------------------
  * replaces utils.clip_gradient (utils.py:51-60) + torch.optim.Adam.step (train_multitask.py:388-389)
@@ -543,6 +550,37 @@ int32_t sn_cider_scores(const int32_t* hyp_tok, const int64_t* hyp_off, int64_t 
                         const int64_t* ref_off, const int64_t* ref_group, int32_t n, double sigma,
                         int32_t max_sentence_len, int64_t max_group_tokens, const int32_t* keys,
                         const int32_t* counts, int64_t capacity, double* scores, double* per_order, void* stream);
+/* sn_cider_scores_rows -- sn_cider_scores for R sampled captions against the references of the corpus the table was
+ *   built from: row r's hypothesis is seqs[r, 1 .. lengths[r]) (int64 [R, ld]; column 0 holds <start>) without a final
+ *   end_token, scored against the references of image img[r] (int64 [R], 0 <= img[r] < n_corpus), with
+ *   ref_len = log(n_corpus) -- the corpus' image count, not R.  ref_off / ref_group are the corpus' CSR (ref_group has
+ *   n_corpus + 1 entries).  max_sentence_len >= ld - 1 and the longest reference; max_group_tokens >= ld - 1 plus the
+ *   largest reference token count of an image used.  The body is sn_cider_scores': with img[r] = r, n_corpus = R and
+ *   the same hypotheses, the scores are bitwise equal. */
+int32_t sn_cider_scores_rows(const int64_t* seqs, int64_t ld, const int64_t* lengths, int64_t R, int32_t end_token,
+                             const int64_t* img, int64_t n_corpus, const int32_t* ref_tok, const int64_t* ref_off,
+                             const int64_t* ref_group, int32_t n, double sigma, int32_t max_sentence_len,
+                             int64_t max_group_tokens, const int32_t* keys, const int32_t* counts, int64_t capacity,
+                             double* scores, void* stream);
+
+/* ---- K12: sampling decode step (sn_sample.cu) ---------------------------------------------------------------------
+ * One draw per live row r of logits [R, ld] (the step's vocabulary projection, V columns), for self-critical training:
+ *   greedy = 0: token = argmax_v (logit_v / temperature + g_v), Gumbel-max;
+ *   greedy = 1: token = argmax_v logit_v;
+ *   ties go to the lowest index.  The noise is computed in double:
+ *     seed_t = seed * 0x9E3779B97F4A7C15 + step        (uint64, wrapping)
+ *     u      = ((hash_u32(seed_t, r, v) >> 8) + 0.5) / 2^24     (hash_u32: the dropout hash of sn_common.cuh)
+ *     g_v    = -log(-log(u))
+ *   seed (uint64) and step (int32, the 1-based draw index) are read from device memory (*seed_dev, *step_dev), so a
+ *   captured CUDA graph of the step draws fresh noise when the counter moves.  The caller advances *step_dev.
+ * Row bookkeeping (rows with done[r] != 0 are skipped; a row's draws go to column `step` of its sequence):
+ *   seqs[r, step] = token (int64 [R, max_len + 2], column 0 = <start>), prev_word[r] = token (int32, the next input),
+ *   logprob[r, step - 1] = logit_token - logsumexp(logits) (temperature 1; float [R, max_len + 1]);
+ *   when token == end_token or step == max_len + 1: done[r] = 1, lengths[r] = step + 1, atomicSub(n_unfinished, 1). */
+int32_t sn_sample_step(const float* logits, int64_t ld, int64_t V, int32_t R, int32_t max_len, int32_t end_token,
+                       double temperature, int32_t greedy, const uint64_t* seed_dev, const int32_t* step_dev,
+                       int32_t* prev_word, int64_t* seqs, int64_t* lengths, float* logprob, int32_t* done,
+                       int32_t* n_unfinished, void* stream);
 
 #ifdef __cplusplus
 }
