@@ -88,6 +88,8 @@ SIGNATURES = {
     "sn_cider_scores": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _D, _I32, _I64, _P, _P, _I64, _P, _P, _P]),
     "sn_cider_scores_rows": (_I32, [_P, _I64, _P, _I64, _I32, _P, _I64, _P, _P, _P, _I32, _D, _I32, _I64, _P, _P, _I64,
                                     _P, _P]),
+    "sn_rouge_l": (_I32, [_P, _P, _I64, _P, _P, _P, _I32, _D, _P, _P]),
+    "sn_rouge_l_rows": (_I32, [_P, _I64, _P, _I64, _I32, _P, _I64, _P, _P, _P, _I32, _D, _P, _P]),
     "sn_sample_step": (_I32, [_P, _I64, _I64, _I32, _I32, _I32, _D, _I32] + [_P] * 9),
 }
 

@@ -50,6 +50,22 @@ def _check_df(err):
         raise SnError("sn_cider_df: " + "; ".join(msg for bit, msg in _DF_ERRORS if err & bit))
 
 
+def _check_samples(seqs, lengths, image_ids, n_img):
+    """The argument checks of ``score_samples`` (ValueError, no device work): returns (R, ld, image ids int64 [R])."""
+    if not isinstance(seqs, torch.Tensor) or seqs.dim() != 2:
+        raise ValueError("seqs must be a 2-D tensor [R, max_len]; got %s" % (
+            tuple(seqs.shape) if isinstance(seqs, torch.Tensor) else type(seqs).__name__,))
+    R, ld = seqs.shape
+    if not isinstance(lengths, torch.Tensor) or tuple(lengths.shape) != (R,):
+        raise ValueError("lengths must be a tensor of shape [%d]" % R)
+    ids = np.asarray(image_ids)
+    if ids.shape != (R,):
+        raise ValueError("%d image ids for %d rows" % (ids.size, R))
+    if R and (not np.issubdtype(ids.dtype, np.integer) or int(ids.min()) < 0 or int(ids.max()) >= n_img):
+        raise ValueError("image ids must be integers in 0..%d" % (n_img - 1))
+    return R, ld, ids.astype(np.int64)
+
+
 def _upload(list_of_references, hypotheses):
     """Checks and packs the corpus and copies it to the device once.  Returns the device views (hyp_tok, hyp_off,
     ref_tok, ref_off, ref_group), max_sentence_len, max_group_tokens, and the host copies of ref_off and ref_group."""
@@ -143,18 +159,7 @@ class CiderD:
         is a host sequence of R corpus positions.  With ``image_ids = range(n_img)`` the scores equal those of
         ``compute_score`` on the same hypotheses bit for bit.  Raises ValueError, before any device work, for a
         ``seqs`` that is not 2-D, mismatched lengths and an image id out of range."""
-        if not isinstance(seqs, torch.Tensor) or seqs.dim() != 2:
-            raise ValueError("seqs must be a 2-D tensor [R, max_len]; got %s" % (
-                tuple(seqs.shape) if isinstance(seqs, torch.Tensor) else type(seqs).__name__,))
-        R, ld = seqs.shape
-        if not isinstance(lengths, torch.Tensor) or tuple(lengths.shape) != (R,):
-            raise ValueError("lengths must be a tensor of shape [%d]" % R)
-        ids = np.asarray(image_ids)
-        if ids.shape != (R,):
-            raise ValueError("%d image ids for %d rows" % (ids.size, R))
-        if R and (not np.issubdtype(ids.dtype, np.integer) or int(ids.min()) < 0 or int(ids.max()) >= self.n_img):
-            raise ValueError("image ids must be integers in 0..%d" % (self.n_img - 1))
-        ids = ids.astype(np.int64)
+        R, ld, ids = _check_samples(seqs, lengths, image_ids, self.n_img)
         dev = self._ref_off.device
         if R == 0:
             return torch.empty(0, dtype=torch.float64, device=dev)

@@ -6,13 +6,15 @@
 with everything id-level done on the device: the loss / top-5 / arg-max come out of the fused softmax kernel instead of
 five passes over the [N, V] logits on the host, and beam search runs for a whole batch of images at once
 (``sample_batch``).  Corpus BLEU over the ids (``bleu.corpus_bleu``, nltk's semantics) and CIDEr-D
-(``cider.corpus_cider``, coco-caption's semantics) run on the device too: ``validate(..., bleu_weights=..., cider=True)``
-adds them to the result, and ``generate``'s captions go to ``bleu.corpus_bleu`` / ``cider.CiderD`` once <start> / <end>
-are stripped.  Ids -> words stays with the caller."""
+(``cider.corpus_cider``) and ROUGE-L (``rouge.corpus_rouge``, both coco-caption's semantics) run on the device too:
+``validate(..., bleu_weights=..., cider=True, rouge=True)`` adds them to the result, and ``generate``'s captions go to
+``bleu.corpus_bleu`` / ``cider.CiderD`` / ``rouge.RougeL`` once <start> / <end> are stripped.  Ids -> words stays
+with the caller."""
 import torch
 
 from .bleu import corpus_bleu
 from .cider import corpus_cider
+from .rouge import corpus_rouge
 from .packing import get_plan
 
 
@@ -22,7 +24,7 @@ def _strip(ids, start, end):
 
 @torch.no_grad()
 def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, attention=None, bleu_weights=None,
-             cider=False):
+             cider=False, rouge=False):
     """``batches`` yields (images_or_features, captions [B,T] int64, lengths, all_captions | None) like the reference's
     data loader (sorted by length, data_loader.py:116-145).  Returns dict(loss, top5 (percent), hypotheses,
     references, n_tokens) with the reference's definitions: loss = token-mean cross entropy averaged over batches
@@ -31,7 +33,8 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
     ``bleu_weights`` (a weight tuple or a list of them): the dict also holds "bleu" =
     ``bleu.corpus_bleu(references, hypotheses, bleu_weights)`` (train_multitask.py:341); every batch then needs its
     all_captions, else ValueError.  ``cider=True``: the dict also holds "cider" = the corpus CIDEr-D
-    ``cider.corpus_cider(references, hypotheses)[0]``, with the same need for all_captions."""
+    ``cider.corpus_cider(references, hypotheses)[0]``, with the same need for all_captions.  ``rouge=True``: the dict
+    also holds "rouge_l" = the corpus ROUGE-L ``rouge.corpus_rouge(references, hypotheses)[0]``, with the same need."""
     was_training = decoder.training
     decoder.eval()
     if encoder is not None:
@@ -42,9 +45,10 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
     tot_tok = 0
     hyps, refs = [], []
     for images, captions, lengths, all_caps in batches:
-        if all_caps is None and (bleu_weights is not None or cider):
+        if all_caps is None and (bleu_weights is not None or cider or rouge):
             decoder.train(was_training)
-            raise ValueError("validate(bleu_weights=... / cider=True) needs the references (all_captions) of every batch")
+            raise ValueError("validate(bleu_weights=... / cider=True / rouge=True) needs the references (all_captions) "
+                             "of every batch")
         feats = encoder(images) if encoder is not None else images
         lengths = [int(l) for l in lengths]
         if att:
@@ -72,6 +76,8 @@ def validate(decoder, batches, start_token, end_token, encoder=None, mode=None, 
         res["bleu"] = corpus_bleu(refs, hyps, bleu_weights)
     if cider:
         res["cider"] = corpus_cider(refs, hyps)[0]
+    if rouge:
+        res["rouge_l"] = corpus_rouge(refs, hyps)[0]
     return res
 
 

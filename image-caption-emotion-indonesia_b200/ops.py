@@ -824,6 +824,31 @@ def cider_scores_rows(seqs, lengths, img, end_token, n_corpus, ref_tok, ref_off,
     return scores
 
 
+def rouge_l(hyp_tok, hyp_off, ref_tok, ref_off, ref_group, max_sentence_len, beta2, out=None):
+    """ROUGE-L per image (sn_rouge_l): float64 [n_img].  Inputs as for ``bleu_counts``; ``beta2`` is the scorer's
+    beta ** 2.  ``out``: a float64 [n_img] CUDA tensor to write the scores into."""
+    n_img = hyp_off.numel() - 1
+    scores = out if out is not None else torch.empty(n_img, dtype=torch.float64, device=hyp_off.device)
+    check(lib().sn_rouge_l(_ptr(_req(hyp_tok, torch.int32)), _ptr(_req(hyp_off, torch.int64)), n_img,
+                           _ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                           _ptr(_req(ref_group, torch.int64)), int(max_sentence_len), float(beta2),
+                           _ptr(_req(scores, torch.float64)), _stream()), "sn_rouge_l")
+    return scores
+
+
+def rouge_l_rows(seqs, lengths, img, end_token, n_corpus, ref_tok, ref_off, ref_group, max_sentence_len, beta2):
+    """ROUGE-L of sampled captions (sn_rouge_l_rows): row r = seqs[r, 1:lengths[r]] without a final end_token, against
+    the references of corpus image img[r].  Returns float64 [R]."""
+    R = seqs.shape[0]
+    scores = torch.empty(R, dtype=torch.float64, device=seqs.device)
+    check(lib().sn_rouge_l_rows(_ptr(_req(seqs, torch.int64)), seqs.stride(0), _ptr(_req(lengths, torch.int64)), R,
+                                int(end_token), _ptr(_req(img, torch.int64)), int(n_corpus),
+                                _ptr(_req(ref_tok, torch.int32)), _ptr(_req(ref_off, torch.int64)),
+                                _ptr(_req(ref_group, torch.int64)), int(max_sentence_len), float(beta2), _ptr(scores),
+                                _stream()), "sn_rouge_l_rows")
+    return scores
+
+
 def sample_step(logits, V, R, max_len, end_token, temperature, greedy, seed_dev, step_dev, prev_word, seqs, lengths,
                 logprob, done, n_unfinished):
     """K12: one sampling-decode draw per live row of ``logits`` (Gumbel-max at ``temperature``, or the arg-max), with

@@ -563,6 +563,31 @@ int32_t sn_cider_scores_rows(const int64_t* seqs, int64_t ld, const int64_t* len
                              int64_t max_group_tokens, const int32_t* keys, const int32_t* counts, int64_t capacity,
                              double* scores, void* stream);
 
+/* ---- K13: ROUGE-L (sn_rouge.cu) -----------------------------------------------------------------------------------
+ * replaces coco-caption's Rouge scorer (pycocoevalcap/rouge/rouge.py, Rouge().compute_score: my_lcs + calc_score) on
+ * integer token ids.  Same CSR inputs as K10; max_sentence_len (longest hypothesis or reference) <= SN_BLEU_MAX_LEN,
+ * else rc < 0 before any launch.  There is no per-image token limit: nothing is staged in shared memory.  Any int32 id
+ * is valid (ids are only compared for equality).
+ * sn_rouge_l -- per image i, with lcs_r = the longest common subsequence of hypothesis i and its reference r (exact,
+ *   bit-parallel), len = the token count, an empty sentence counting as one token that only another empty sentence
+ *   shares ("".split(" ") == [""]):
+ *     p = max_r lcs_r / len_hyp,  r = max_r (lcs_r / len_ref_r),
+ *     scores[i] = ((1 + beta2) * p * r) / (r + beta2 * p) if p != 0 and r != 0, else 0,
+ *   every operation one correctly rounded float64 operation in that order (no FMA contraction), so the scores equal
+ *   the scorer's bit for bit when beta2 is its beta**2 (1.2 ** 2).  No atomics: run-to-run identical.  An image whose
+ *   sizes exceed the declared maximum, or without references, gets NaN.  The corpus score is the mean of scores[].
+ * sn_rouge_l_rows -- the same body for R sampled captions against the references of a corpus (sn_cider_scores_rows'
+ *   layout): row r's hypothesis is seqs[r, 1 .. lengths[r]) (int64 [R, ld]; column 0 holds <start>) without a final
+ *   end_token, scored against the references of image img[r] (int64 [R], 0 <= img[r] < n_corpus; NaN otherwise).
+ *   ld - 1 <= max_sentence_len.  With img[r] = r and the same hypotheses, the scores equal sn_rouge_l's bit for bit. */
+int32_t sn_rouge_l(const int32_t* hyp_tok, const int64_t* hyp_off, int64_t n_img, const int32_t* ref_tok,
+                   const int64_t* ref_off, const int64_t* ref_group, int32_t max_sentence_len, double beta2,
+                   double* scores, void* stream);
+int32_t sn_rouge_l_rows(const int64_t* seqs, int64_t ld, const int64_t* lengths, int64_t R, int32_t end_token,
+                        const int64_t* img, int64_t n_corpus, const int32_t* ref_tok, const int64_t* ref_off,
+                        const int64_t* ref_group, int32_t max_sentence_len, double beta2, double* scores,
+                        void* stream);
+
 /* ---- K12: sampling decode step (sn_sample.cu) ---------------------------------------------------------------------
  * One draw per live row r of logits [R, ld] (the step's vocabulary projection, V columns), for self-critical training:
  *   greedy = 0: token = argmax_v (logit_v / temperature + g_v), Gumbel-max;
